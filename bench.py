@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path (N>1: launched by torchrun, one rank/GPU)
   python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host CPU cores (oracle port)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A bench "step" = ONE complete closed-loop rollout of the per-GPU workload (BASELINE config 3: 16 scenes x 32 rollouts,
 128 agents, 1024 polylines x 20 nodes, 40 traffic lights, 11-step history): 90 policy iterations of which the 80
@@ -52,7 +53,49 @@ def parse():
                          "(--scenes scenes per GPU, default 64; dropout 0) - prints its own JSON line")
     ap.add_argument("--rule-checks", action="store_true",
                     help="also run the logging-only TrafficRuleChecker checks (collision, road edge, ...) every step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32, or "
+                         "float64 where the output is), at most 64 MB in all: larger outputs are cut to a fixed, seeded "
+                         "sample of rows. Inputs depend only on the arguments, so two builds can be compared file by file")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path, not to --impl reference")
+    return args
+
+
+DUMP_BYTES = 64 * 10**6  # 64 MB, npy headers included
+
+
+def dump_outputs(out_dir, whole, rows=None, seed=0):
+    """Write every tensor of `whole` and `rows` to out_dir/<name>.npy: float64 stays float64, everything else (fp32,
+    fp16, bool, int) becomes float32. The tensors of `rows` share their leading dimension; if the files would exceed
+    DUMP_BYTES in all, those tensors are cut to the same rows, drawn by a generator seeded with `seed` and kept in
+    ascending order, so the sample depends only on the shapes. Returns a short description for the log."""
+    import numpy as np
+    rows = rows or {}
+
+    def host(t):
+        return t.detach().to("cpu", torch.float64 if t.dtype == torch.float64 else torch.float32)
+
+    whole = {k: host(v) for k, v in whole.items()}
+    nbytes = lambda ts: sum(t.numel() * t.element_size() for t in ts)  # noqa: E731
+    budget = DUMP_BYTES - nbytes(whole.values()) - 256 * (len(whole) + len(rows))  # npy headers
+    n = next(iter(rows.values())).shape[0] if rows else 0
+    per_row = sum(v[0].numel() * (8 if v.dtype == torch.float64 else 4) for v in rows.values())
+    keep = min(n, budget // per_row) if rows else 0
+    if rows and keep < 1:
+        raise ValueError(f"--dump-outputs: the outputs do not fit {DUMP_BYTES / 1e6:.0f} MB even at one row")
+    sel = None
+    if keep < n:
+        sel = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+    out = dict(whole, **{k: host(v if sel is None else v[sel.to(v.device)]) for k, v in rows.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.numpy())
+    what = f"{len(out)} arrays, {nbytes(out.values()) / 1e6:.1f} MB"
+    return what if sel is None else what + f"; {keep} of {n} rows of {', '.join(rows)} (seed {seed})"
 
 
 class ClockSampler:
@@ -477,6 +520,9 @@ def run_sweep(args):
         t_val = timed(lambda: sweep(resident), args.steps)
     launches = (ops.LAUNCHES - l0) + args.steps * n_batches * eng.graph_steps * eng.launches_per_step
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:  # the last sweep's gathered trajectories, one row per (scene, rollout)
+        print("dump-outputs:", dump_outputs(args.dump_outputs, {}, dict(pred_pose=og.store.flatten(0, 2))),
+              file=sys.stderr, flush=True)
     units = total * R * N_COUNTED
     value = units * args.steps / t_val
 
@@ -590,6 +636,11 @@ def run_ours(args):
         t_loop = timed(loop_step, args.steps)
     launches = args.steps * eng.graph_steps * eng.launches_per_step + (ops.LAUNCHES - l0)  # graph replays + eager launches
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:
+        # eng.results() is what the last eng.run() returned (its buffers are not touched again before e2e below);
+        # joint_pose is pred_pose viewed per scene, so it is left out
+        res = {k: v for k, v in eng.results().items() if k != "joint_pose"}
+        print("dump-outputs:", dump_outputs(args.dump_outputs, {}, res), file=sys.stderr, flush=True)
     units = world * n_sc * args.rollouts * N_COUNTED
     value = units * args.steps / t_loop
 
@@ -711,9 +762,13 @@ def run_train(args):
     if world > 1:
         ts.data_parallel()  # gradients averaged with one NCCL all-reduce per step (inside the timed region)
 
+    last = {}
+
     def step():
         ts.zero_grad()
         out = ts.step(batch)
+        if args.dump_outputs:
+            last["out"] = out
         return float(out["loss"].detach())  # device -> host read of the step's result
 
     def barrier():
@@ -739,6 +794,12 @@ def run_train(args):
     t = float(tt)
     phases = ts.timings_ms()
     peak_gb = torch.cuda.max_memory_allocated() / 2 ** 30
+    if args.dump_outputs and rank == 0:  # the last step's losses and trajectories, and the gradients it left
+        out = last["out"]
+        whole = {k: v for k, v in out.items() if torch.is_tensor(v) and k not in ("pred_pose", "pred_valid")}
+        whole.update({f"grad.{k}": p.grad for k, p in ts.params.items() if p.grad is not None})
+        rows = dict(pred_pose=out["pred_pose"], pred_valid=out["pred_valid"])
+        print("dump-outputs:", dump_outputs(args.dump_outputs, whole, rows), file=sys.stderr, flush=True)
     if rank != 0:
         dist.barrier()
         dist.destroy_process_group()
