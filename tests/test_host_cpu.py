@@ -64,6 +64,28 @@ def test_fused_attention_weights_reproduce_the_reference_formulation():
         assert float((out - ref).abs().max()) < 1e-5 * float(ref.abs().max()), interleaved
 
 
+def test_knarpe_core_reference_composes_to_attention_rpe():
+    """tests/_knarpe_ref.py (the float64 core the GPU stress tests compare against), composed with fuse_attention's
+    packed projections, reproduces the oracle's AttentionRPE in float64: masked neighbours, an all-masked token, both
+    model widths. The only difference is fuse_attention's fp32 rounding of the packed weights (2^-24 relative)."""
+    import _knarpe_ref as KR
+    for d, K in ((128, 9), (256, 5)):
+        B, S = 2, 6
+        g = torch.Generator().manual_seed(d + K)
+        shapes = {"in_proj_weight": (3 * d, d), "in_proj_bias": (3 * d,), "out_proj_weight": (d, d),
+                  "out_proj_bias": (d,), "linear_rpe.weight": (2 * d, d), "linear_rpe.bias": (2 * d,)}
+        P = {f"a.{k}": v.double() for k, v in params.rand_like_state_dict(shapes, 7).items()}
+        src, tgt = torch.randn(B, S, d, generator=g).double(), torch.randn(B, S, K, d, generator=g).double()
+        mask = torch.rand(B, S, K, generator=g) < 0.3
+        mask[1, 2] = True
+        rel = torch.cat([torch.randn(B, S, K, 2, generator=g) * 30, torch.randn(B, S, K, 1, generator=g) * 2], -1).double()
+        ref = O.attention_rpe(P, "a", src, tgt, mask, O.pose_emb_xy_yaw(rel[..., :2], rel[..., 2], d), H)
+        out = KR.attention_from_core(fuse_attention(P, "a", d), src, tgt, mask, rel)
+        assert out.dtype == torch.float64
+        assert float((out - ref).abs().max()) < 1e-6 * float(ref.abs().max()), d
+        assert float(out[1, 2].abs().max()) == 0.0
+
+
 def test_rollout_buffer_layout_and_log_prob():
     """RolloutBuffer of the rollout-level drop-in (utils/buffer.py:103-146): joint-future flattening and the navigation
     log-probability average, on hand-made tensors (no GPU)."""

@@ -1,10 +1,9 @@
 """GPU parity tests: every CUDA kernel (called through the C ABI via ops.*) against the CPU oracle and against
 the golden vectors produced by the real reference. Tolerances are written next to each check."""
-import math
-
 import pytest
 import torch
 
+import _knarpe_ref as KR
 from oracle import tb_oracle as O
 from trafficbotsv1_5_b200 import config, params
 
@@ -619,22 +618,12 @@ def test_knarpe_attn_backward_vs_autograd(B, S, T0, K0, T1, K1, div1):
     rel = torch.cat([(torch.rand(B, S, K, 2, generator=g) * 2 - 1) * 100, (torch.rand(B, S, K, 1, generator=g) * 2 - 1) * 3], -1)
     d_out = torch.randn(M, 5 * d, generator=g)
 
-    # float64 autograd reference of the core op
+    # float64 autograd reference of the core op (tests/_knarpe_ref.py)
     qd, ud, k0d = q.double().requires_grad_(), u.double().requires_grad_(), kv0.double().requires_grad_()
     k1d = kv1.double().requires_grad_() if K1 else None
-    rows0 = k0d.view(B, T0, 2 * d)[torch.arange(B)[:, None, None], idx[..., :K0]]                  # [B,S,K0,2d]
-    rows = rows0 if not K1 else torch.cat(
-        [rows0, k1d.view(B // div1, T1, 2 * d)[(torch.arange(B) // div1)[:, None, None], idx[..., K0:]]], 2)
-    e = O.pose_emb_xy_yaw(rel[..., :2].double(), rel[..., 2].double(), d)                          # [B,S,K,d]
-    kk, vv = rows[..., :d].reshape(M, K, H, d // H), rows[..., d:].reshape(M, K, H, d // H)
-    lg = torch.einsum("mhc,mkhc->mhk", qd.view(M, H, d // H), kk) + torch.einsum("mhc,mkc->mhk", ud.view(M, H, d), e.view(M, K, d))
-    msk = inv.view(M, 1, K)
-    none = inv.view(M, K).all(-1)
-    p = torch.softmax((lg * math.log(2.0)).masked_fill(msk, -float("inf")).masked_fill(none[:, None, None], 0.0), -1)
-    p = p.masked_fill(msk, 0.0)
-    ov = torch.einsum("mhk,mkhc->mhc", p, vv).reshape(M, d)
-    z = torch.einsum("mhk,mkc->mhc", p, e.view(M, K, d)).reshape(M, H * d)
-    out = torch.cat([ov, z], -1).masked_fill(none[:, None], 0.0)
+    rows = KR.gather_rows(k0d, T0, 1, K0, idx, B, k1d, T1, div1)
+    ov, z, _ = KR.knarpe_core(qd, ud, rows, inv, rel)
+    out = torch.cat([ov, z], -1)
     out.backward(d_out.double())
     # the forward kernel agrees with this reference (sanity of the test itself)
     dv = lambda t: None if t is None else t.to(DEV).contiguous()  # noqa: E731
