@@ -349,6 +349,21 @@ int tb_dyn_step_ex(const float* act_branch, const uint8_t* ag_type, const float*
                    int n_mp, int n_node, float thresh_lane, float thresh_edge, float cos_rot, const int* d_step, int B,
                    int A, int W, int T, uint8_t* hist_valid, float* hist_pose, float* hist_motion, uint8_t* pred_valid,
                    float* pred_pose, float* pred_motion, uint8_t* o_outside, uint8_t* o_reached, void* stream);
+/* tb_dyn_step_ex + the player override of Dynamics.update_ag (utils/dynamics.py:96-99, waymo_motion.py:206-217):
+ *   player_valid [B*A] u8 (optional, NULL = no player; then the bits of tb_dyn_step_ex), player_action [B*A, T, 2]
+ *   physical (acc m/s^2, yaw rate rad/s), required with player_valid. Step s of a valid, typed agent with
+ *   player_valid set uses player_action[.., s-1, :] instead of the tanh-scaled action head; pred_* record that
+ *   prediction, then teacher forcing and the outside-map / destination checks run unchanged. */
+int tb_dyn_step_player(const float* act_branch, const uint8_t* ag_type, const float* max_acc,
+                       const float* max_yaw_rate, float dt, uint8_t* valid, uint8_t* disabled, uint8_t* navi_invalid,
+                       uint8_t* dest_reached, float* pose, float* motion, const uint8_t* gt_valid, const float* gt_pose,
+                       const float* gt_motion, const uint8_t* tf_mask, int n_gt, int sc_div, const float* boundary,
+                       const int32_t* dest_idx, const float* mp_pos, const float* mp_dirn,
+                       const uint8_t* mp_node_invalid, const uint8_t* mp_kind, int n_mp, int n_node, float thresh_lane,
+                       float thresh_edge, float cos_rot, const int* d_step, int B, int A, int W, int T,
+                       uint8_t* hist_valid, float* hist_pose, float* hist_motion, uint8_t* pred_valid, float* pred_pose,
+                       float* pred_motion, uint8_t* o_outside, uint8_t* o_reached, const uint8_t* player_valid,
+                       const float* player_action, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Fused MLP chain (csrc/mlp_chain.cu): a sequence of dense layers over 128-row tiles with every intermediate kept on

@@ -101,6 +101,7 @@ struct DynArgs {
   float cos_rot; const int* d_step; int n_tot; int A; int W; int T;
   uint8_t* hist_valid; float* hist_pose; float* hist_motion; uint8_t* pred_valid; float* pred_pose; float* pred_motion;
   uint8_t* o_outside; uint8_t* o_reached;  // optional [B,A,T]: outside_map_this_step / dest_reached_this_step (buffer.py:57-60)
+  const uint8_t* player_valid; const float* player_action;  // optional [B*A] / [B*A,T,2]: player override (dynamics.py:96-99)
 };
 
 __global__ void __launch_bounds__(128) dyn_step_kernel(DynArgs p) {
@@ -118,6 +119,11 @@ __global__ void __launch_bounds__(128) dyn_step_kernel(DynArgs p) {
   if (v_old && type >= 0) {
     acc = tanhf(p.act_branch[(size_t)i * 6 + type * 2 + 0]) * p.max_acc[type];
     yr = tanhf(p.act_branch[(size_t)i * 6 + type * 2 + 1]) * p.max_yaw[type];
+    if (p.player_valid && p.player_valid[i]) {  // the player's physical action replaces the policy's (dynamics.py:96-99)
+      const size_t o = ((size_t)i * p.T + (s - 1)) * 2;
+      acc = p.player_action[o];
+      yr = p.player_action[o + 1];
+    }
   }
   // ---- MultiPathPP.update (dynamics.py:248-274), same operation order as the reference (no FMA contraction)
   float x = p.pose[(size_t)i * 3], y = p.pose[(size_t)i * 3 + 1], w = p.pose[(size_t)i * 3 + 2];
@@ -307,19 +313,22 @@ extern "C" int tb_tl_featurize(const uint8_t* hist_tl, const uint8_t* tl_invalid
   return tb_tl_featurize_ex(hist_tl, tl_invalid, d_step, 0, B, TL, W, attr_out, lda, row_invalid, stream);
 }
 
-extern "C" int tb_dyn_step_ex(const float* act_branch, const uint8_t* ag_type, const float* max_acc,
-                              const float* max_yaw_rate, float dt, uint8_t* valid, uint8_t* disabled, uint8_t* navi_invalid,
-                              uint8_t* dest_reached, float* pose, float* motion, const uint8_t* gt_valid,
-                              const float* gt_pose, const float* gt_motion, const uint8_t* tf_mask, int n_gt, int sc_div,
-                              const float* boundary, const int32_t* dest_idx, const float* mp_pos, const float* mp_dirn,
-                              const uint8_t* mp_node_invalid, const uint8_t* mp_kind, int n_mp, int n_node,
-                              float thresh_lane, float thresh_edge, float cos_rot, const int* d_step, int B, int A, int W,
-                              int T, uint8_t* hist_valid, float* hist_pose, float* hist_motion, uint8_t* pred_valid,
-                              float* pred_pose, float* pred_motion, uint8_t* o_outside, uint8_t* o_reached, void* stream) {
+extern "C" int tb_dyn_step_player(const float* act_branch, const uint8_t* ag_type, const float* max_acc,
+                                  const float* max_yaw_rate, float dt, uint8_t* valid, uint8_t* disabled,
+                                  uint8_t* navi_invalid, uint8_t* dest_reached, float* pose, float* motion,
+                                  const uint8_t* gt_valid, const float* gt_pose, const float* gt_motion,
+                                  const uint8_t* tf_mask, int n_gt, int sc_div, const float* boundary,
+                                  const int32_t* dest_idx, const float* mp_pos, const float* mp_dirn,
+                                  const uint8_t* mp_node_invalid, const uint8_t* mp_kind, int n_mp, int n_node,
+                                  float thresh_lane, float thresh_edge, float cos_rot, const int* d_step, int B, int A,
+                                  int W, int T, uint8_t* hist_valid, float* hist_pose, float* hist_motion,
+                                  uint8_t* pred_valid, float* pred_pose, float* pred_motion, uint8_t* o_outside,
+                                  uint8_t* o_reached, const uint8_t* player_valid, const float* player_action,
+                                  void* stream) {
   if (!act_branch || !ag_type || !max_acc || !max_yaw_rate || !valid || !disabled || !navi_invalid || !dest_reached ||
       !pose || !motion || !gt_valid || !gt_pose || !gt_motion || !tf_mask || !boundary || !dest_idx || !mp_pos ||
       !mp_dirn || !mp_node_invalid || !mp_kind || !d_step || !hist_valid || !hist_pose || !hist_motion || !pred_valid ||
-      !pred_pose || !pred_motion)
+      !pred_pose || !pred_motion || (player_valid && !player_action))
     return TB_ERR_NULL;
   if (B <= 0 || A <= 0 || W <= 0 || T <= 0 || n_gt <= 0 || sc_div <= 0 || n_mp <= 0 || n_node <= 0)
     return TB_ERR_BAD_SHAPE;
@@ -333,10 +342,26 @@ extern "C" int tb_dyn_step_ex(const float* act_branch, const uint8_t* ag_type, c
   p.n_node = n_node; p.thresh_lane = thresh_lane; p.thresh_edge = thresh_edge; p.cos_rot = cos_rot; p.d_step = d_step;
   p.n_tot = B * A; p.A = A; p.W = W; p.T = T; p.hist_valid = hist_valid; p.hist_pose = hist_pose;
   p.hist_motion = hist_motion; p.pred_valid = pred_valid; p.pred_pose = pred_pose; p.pred_motion = pred_motion;
-  p.o_outside = o_outside; p.o_reached = o_reached;
+  p.o_outside = o_outside; p.o_reached = o_reached; p.player_valid = player_valid; p.player_action = player_action;
   dyn_step_kernel<<<(p.n_tot + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(p);
   TB_CHECK_LAUNCH();
   return TB_OK;
+}
+
+extern "C" int tb_dyn_step_ex(const float* act_branch, const uint8_t* ag_type, const float* max_acc,
+                              const float* max_yaw_rate, float dt, uint8_t* valid, uint8_t* disabled, uint8_t* navi_invalid,
+                              uint8_t* dest_reached, float* pose, float* motion, const uint8_t* gt_valid,
+                              const float* gt_pose, const float* gt_motion, const uint8_t* tf_mask, int n_gt, int sc_div,
+                              const float* boundary, const int32_t* dest_idx, const float* mp_pos, const float* mp_dirn,
+                              const uint8_t* mp_node_invalid, const uint8_t* mp_kind, int n_mp, int n_node,
+                              float thresh_lane, float thresh_edge, float cos_rot, const int* d_step, int B, int A, int W,
+                              int T, uint8_t* hist_valid, float* hist_pose, float* hist_motion, uint8_t* pred_valid,
+                              float* pred_pose, float* pred_motion, uint8_t* o_outside, uint8_t* o_reached, void* stream) {
+  return tb_dyn_step_player(act_branch, ag_type, max_acc, max_yaw_rate, dt, valid, disabled, navi_invalid, dest_reached,
+                            pose, motion, gt_valid, gt_pose, gt_motion, tf_mask, n_gt, sc_div, boundary, dest_idx, mp_pos,
+                            mp_dirn, mp_node_invalid, mp_kind, n_mp, n_node, thresh_lane, thresh_edge, cos_rot, d_step, B,
+                            A, W, T, hist_valid, hist_pose, hist_motion, pred_valid, pred_pose, pred_motion, o_outside,
+                            o_reached, nullptr, nullptr, stream);
 }
 
 extern "C" int tb_dyn_step(const float* act_branch, const uint8_t* ag_type, const float* max_acc,

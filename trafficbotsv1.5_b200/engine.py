@@ -121,7 +121,11 @@ class RolloutEngine:
         self.graph_steps = 0  # graph replays of the last run() (bench.py: launch accounting)
         self._by_shape = {}  # shape -> (state, static, navi, graphs, launches per step) of recently used batch shapes
         self._static = self._navi = None
-        self._graph = None   # (graph for odd steps, graph for even steps): the TL branch is double-buffered
+        # player mode -> (graph for odd steps, graph for even steps): the TL branch is double-buffered, and a batch with
+        # "player/valid" launches the dynamics with the player override (tb_dyn_step_player), so it has graphs of its own
+        self._graphs = {}
+        self._players = False  # the prepared batch has player-controlled agents
+        self._t = None       # current time of step-by-step stepping (begin / step); None: not begun
         self._host_step = 1  # parity source for eager _step calls
         self._shape = None
         self._side = torch.cuda.Stream(device=self.dev)  # traffic-light branch runs beside the agent front-end
@@ -133,6 +137,11 @@ class RolloutEngine:
         self.thresh_lane = float(one * 50 * (1 - torch.zeros(1) * 0.8))
         self.thresh_edge = float(one * 50 * (1 - one * 0.8))
         self.cos_rot = float(torch.tensor(np.cos(np.deg2rad(30)), dtype=torch.float32))
+
+    @property
+    def _graph(self):
+        """Step graphs of the prepared batch's shape and player mode (None until captured)."""
+        return self._graphs.get(self._players)
 
     # ---------------------------------------------------------------------------------------------- scene encoding
     def encode_scenes(self, batch: Dict[str, Tensor]) -> dict:
@@ -262,7 +271,17 @@ class RolloutEngine:
         st["gt_valid"].copy_(gt_valid)
         st["gt_pose"].copy_(g("sc/ag_pose"))
         st["gt_motion"].copy_(g("sc/ag_motion"))
-        st["tf_mask"].copy_(teacher_forcing_mask(gt_valid, *self.tf_steps))
+        tf = teacher_forcing_mask(gt_valid, *self.tf_steps)
+        if "tf/forcing_agent" in batch:  # log replay of whole agents (teacher_forcing.py:87-92, as TrainStep)
+            tf = tf | (g("tf/forcing_agent")[:, :, None] & gt_valid)
+        st["tf_mask"].copy_(tf)
+        if "player/valid" in batch:  # [n_sc, R, A(, T, 2)] after _player_inputs / _compact
+            B, A = st["B"], st["A"]
+            if "player_valid" not in st:  # allocated on first use; the player-mode graphs point at these buffers
+                st["player_valid"] = torch.zeros(B, A, dtype=torch.uint8, device=dev)
+                st["player_action"] = torch.zeros(B, A, self.T, 2, device=dev)
+            st["player_valid"].copy_(g("player/valid").reshape(B, A))
+            st["player_action"].copy_(g("player/action").reshape(B, A, self.T, 2))
         tl_gt = g("sc/tl_state")
         st["gt_tl"].copy_(tl_gt if self.tl_per_scene else rep(tl_gt))
         st["boundary"].copy_(g("map/boundary"))
@@ -360,7 +379,7 @@ class RolloutEngine:
         m, lib = self.model, L.load()
         dy = self.dyn
         order = ("veh", "ped", "cyc")
-        L.check(lib.tb_dyn_step_ex(
+        args = (
             L.ptr(act), L.ptr(st["ag_type"]), ops.host_f3([dy[k]["max_acc"] for k in order]),
             ops.host_f3([dy[k]["max_yaw_rate"] for k in order]), dy["dt"], L.ptr(st["valid"]), L.ptr(st["disabled"]),
             L.ptr(ops._u8(st["navi_invalid"])), L.ptr(st["dest_reached"]), L.ptr(st["pose"]), L.ptr(st["motion"]),
@@ -369,7 +388,12 @@ class RolloutEngine:
             L.ptr(st["mp_node_invalid"]), L.ptr(st["mp_kind"]), st["n_mp"], st["n_node"], self.thresh_lane,
             self.thresh_edge, self.cos_rot, L.ptr(st["d_step"]), st["B"], st["A"], m.W, self.T, L.ptr(st["hist_valid"]),
             L.ptr(st["hist_pose"]), L.ptr(st["hist_motion"]), L.ptr(st["pred_valid"]), L.ptr(st["pred_pose"]),
-            L.ptr(st["pred_motion"]), L.ptr(st.get("fb_outside")), L.ptr(st.get("fb_reached")), L.stream()), "tb_dyn_step_ex")
+            L.ptr(st["pred_motion"]), L.ptr(st.get("fb_outside")), L.ptr(st.get("fb_reached")))
+        if self._players:  # the player's plan column s-1 replaces the action head of player agents (dynamics.py:96-99)
+            L.check(lib.tb_dyn_step_player(*args, L.ptr(st["player_valid"]), L.ptr(st["player_action"]), L.stream()),
+                    "tb_dyn_step_player")
+        else:
+            L.check(lib.tb_dyn_step_ex(*args, L.stream()), "tb_dyn_step_ex")
         if join is not None:
             torch.cuda.current_stream().wait_stream(join)  # TL feedback of this step applied, TL tokens of the next ready
         if self.rule_checks:
@@ -464,7 +488,36 @@ class RolloutEngine:
 
     # ---------------------------------------------------------------------------------------------- public API
     _AGENT_KEYS = {"sc/ag_valid": 1, "sc/ag_pose": 1, "sc/ag_motion": 1, "sc/ag_attr": 1, "ref/ag_type": 1, "ref/ag_size": 1,
-                   "ag_latent": 2, "ag_latent_valid": 1, "ag_navi_valid": 1, "ref/ag_role": 1}
+                   "ag_latent": 2, "ag_latent_valid": 1, "ag_navi_valid": 1, "ref/ag_role": 1, "tf/forcing_agent": 1,
+                   "player/valid": 2, "player/action": 2}  # player arrays are per rollout after _player_inputs
+
+    def _player_inputs(self, batch: Dict[str, Tensor]) -> Dict[str, Tensor]:
+        """Check the optional caller-control keys and bring the player arrays to the per-rollout layout:
+        "player/valid" [n_sc, (R,) A] bool, "player/action" [n_sc, (R,) A, step_end, 2] (physical units: m/s^2, rad/s;
+        step s reads column s-1), "tf/forcing_agent" [n_sc, A] bool. Raises ValueError on wrong shapes / dtypes and
+        non-finite actions."""
+        n_sc, A, _ = batch["sc/ag_valid"].shape
+        R, T = self.R, self.T
+        fa = batch.get("tf/forcing_agent")
+        if fa is not None and (fa.dtype != torch.bool or tuple(fa.shape) != (n_sc, A)):
+            raise ValueError(f"tf/forcing_agent: expected bool [{n_sc}, {A}], got {fa.dtype} {tuple(fa.shape)}")
+        if "player/valid" not in batch:
+            if "player/action" in batch:
+                raise ValueError("player/action without player/valid")
+            return batch
+        pv, pa = batch["player/valid"], batch.get("player/action")
+        if pv.dtype != torch.bool or tuple(pv.shape) not in ((n_sc, A), (n_sc, R, A)):
+            raise ValueError(f"player/valid: expected bool [{n_sc}, ({R},) {A}], got {pv.dtype} {tuple(pv.shape)}")
+        if pa is None:
+            raise ValueError("player/valid needs player/action (begin() starts from a zero plan)")
+        if not pa.is_floating_point() or tuple(pa.shape) not in ((n_sc, A, T, 2), (n_sc, R, A, T, 2)):
+            raise ValueError(f"player/action: expected float [{n_sc}, ({R},) {A}, {T}, 2], got {pa.dtype} {tuple(pa.shape)}")
+        if not bool(torch.isfinite(pa).all()):
+            raise ValueError("player/action holds non-finite values")
+        out = dict(batch)
+        out["player/valid"] = pv if pv.dim() == 3 else pv[:, None].expand(-1, R, -1)
+        out["player/action"] = (pa if pa.dim() == 5 else pa[:, None].expand(-1, R, -1, -1, -1)).float()
+        return out
 
     def _compact(self, batch: Dict[str, Tensor]) -> Dict[str, Tensor]:
         """Drop the agent slots that are invalid at every ground-truth step in all scenes of the batch (see
@@ -502,8 +555,11 @@ class RolloutEngine:
         return out
 
     def prepare(self, batch: Dict[str, Tensor], static: Optional[dict] = None) -> dict:
-        """Upload a batch of scenes, encode them (unless `static` is given) and build the step graph."""
-        batch = self._compact(batch)
+        """Upload a batch of scenes, encode them (unless `static` is given) and build the step graph.
+        Optional keys: "player/valid" + "player/action" (an open-loop plan for chosen agents, see `_player_inputs`)
+        and "tf/forcing_agent" (log replay: these agents follow their ground truth wherever it is valid)."""
+        batch = self._compact(self._player_inputs(batch))
+        self._players, self._t = "player/valid" in batch, None
         n_sc, A, n_gt = batch["sc/ag_valid"].shape
         n_tl = batch["sc/tl_valid"].shape[1]
         _, n_mp, n_node = batch["sc/mp_valid"].shape
@@ -513,25 +569,25 @@ class RolloutEngine:
             # state buffers, scene tensors and step graphs are kept per shape (a few, LRU): with agent compaction
             # consecutive batches may differ in the number of agent slots, and a re-capture costs ~0.3 s
             if self._shape is not None:
-                self._by_shape[self._shape] = (self._st, self._static, self._navi, self._graph,
+                self._by_shape[self._shape] = (self._st, self._static, self._navi, self._graphs,
                                                getattr(self, "launches_per_step", 0))
                 while len(self._by_shape) > 3:
                     self._by_shape.pop(next(iter(self._by_shape)))
             if shape in self._by_shape:
-                self._st, self._static, self._navi, self._graph, self.launches_per_step = self._by_shape.pop(shape)
+                self._st, self._static, self._navi, self._graphs, self.launches_per_step = self._by_shape.pop(shape)
             else:
-                self._st, self._static, self._navi, self._graph = self._alloc(*shape), None, None, None
+                self._st, self._static, self._navi, self._graphs = self._alloc(*shape), None, None, {}
             self._shape = shape
         st = self._st
         self._load_state(st, batch)
         new_static = static if static is not None else self.encode_scenes(batch)
         new_navi = self.model.navi_static(new_static["mp"], st["dest_idx"], self.R)
         self.model.latent_static(new_navi, st)
-        if self._graph is not None and _same_layout((self._static, self._navi), (new_static, new_navi)):
-            # same shapes as the captured step graph: refresh the scene tensors in place, keep the graph
+        if self._graphs and _same_layout((self._static, self._navi), (new_static, new_navi)):
+            # same shapes as the captured step graphs: refresh the scene tensors in place, keep the graphs
             _copy_tree((self._static, self._navi), (new_static, new_navi))
         else:
-            self._static, self._navi, self._graph = new_static, new_navi, None
+            self._static, self._navi, self._graphs = new_static, new_navi, {}
         self._s0 = self._invariant_steps(st) if (self.warm_dedup and self.tl_per_scene) else 0
         self._warm = self._build_warm(st, self._static) if self._s0 else None
         return st
@@ -543,30 +599,15 @@ class RolloutEngine:
             raise ValueError(f"run(n_steps={n_steps}): the engine was built with step_end={self.T}")
         warm = self._s0 > 0 and record is None
         done = 0
+        self._t = None
         if self.use_graph and record is None:
-            if self._graph is None:
-                self._reset(st)
-                s = torch.cuda.Stream()
-                s.wait_stream(torch.cuda.current_stream())
-                with torch.cuda.stream(s):
-                    self._step(st, self._static, self._navi)  # warm-up (allocator, lazy module load)
-                torch.cuda.current_stream().wait_stream(s)
-                self._reset(st)
-                graphs = []
-                for parity in (1, 0):  # first step is odd
-                    n0 = ops.LAUNCHES
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        self._step(st, self._static, self._navi, parity=parity)
-                    self.launches_per_step = ops.LAUNCHES - n0
-                    graphs.append(g)
-                self._graph = (graphs[0], graphs[1])  # indexed by (step + 1) % 2: odd steps first
+            graph = self._captured_graph()
             self._reset(st, tl_prologue=not warm)
             if warm:  # rollout-invariant warm-start steps: encoders once per scene, all steps in one batch
                 done = self._warm_steps(st, self._static, self._navi, n_steps)
             self.graph_steps = n_steps - done
             for s_ in range(done + 1, n_steps + 1):
-                self._graph[(s_ + 1) % 2].replay()
+                graph[(s_ + 1) % 2].replay()
         else:
             self._reset(st, tl_prologue=not warm)
             if warm:
@@ -581,6 +622,101 @@ class RolloutEngine:
                     record(s_, aux)
         return self.results()
 
+    def _captured_graph(self):
+        """The (odd step, even step) graphs of the prepared batch's shape and player mode, captured on first use."""
+        if self._graph is None:
+            st = self._st
+            self._reset(st)
+            s = torch.cuda.Stream()
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                self._step(st, self._static, self._navi)  # warm-up (allocator, lazy module load)
+            torch.cuda.current_stream().wait_stream(s)
+            self._reset(st)
+            graphs = []
+            for parity in (1, 0):  # first step is odd
+                n0 = ops.LAUNCHES
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._step(st, self._static, self._navi, parity=parity)
+                self.launches_per_step = ops.LAUNCHES - n0
+                graphs.append(g)
+            self._graphs[self._players] = (graphs[0], graphs[1])  # indexed by (step + 1) % 2: odd steps first
+        return self._graph
+
+    # ---------------------------------------------------------------------------------------------- step by step
+    def begin(self, batch: Dict[str, Tensor], static: Optional[dict] = None) -> Dict[str, Tensor]:
+        """Step-by-step stepping for closed-loop planners: `prepare` the batch, reset to time 0 and, when warm-start
+        de-duplication applies, run its rollout-invariant steps 1 .. S0 (every valid agent is teacher-forced there, so a
+        player only changes its own pred_* of those steps; they use the columns of batch["player/action"], a zero plan
+        when the key is absent). Returns the observation at the current time t (see `step`)."""
+        if "player/valid" in batch and "player/action" not in batch:
+            n_sc, A, _ = batch["sc/ag_valid"].shape
+            batch = dict(batch, **{"player/action": torch.zeros(n_sc, A, self.T, 2)})
+        self.prepare(batch, static)
+        st = self._st
+        if self.use_graph:
+            self._captured_graph()
+        warm = self._s0 > 0
+        self._reset(st, tl_prologue=not warm)
+        self._t = self._warm_steps(st, self._static, self._navi, self.T) if warm else 0
+        self.graph_steps = 0
+        return self._observe()
+
+    def step(self, player_action: Optional[Tensor] = None) -> Dict[str, Tensor]:
+        """Policy step t + 1 of a rollout started with `begin`. `player_action` [n_sc, (R,) A, 2] (caller's agent order,
+        physical units) becomes column t of the plan (a plain async copy), so the agents of batch["player/valid"]
+        follow it in this step; None keeps the plan's column. Replays one step graph and returns the observation at
+        the new time: dict(t=int, valid [n_sc*R, A] bool, pose / motion [n_sc*R, A, 3]) on the device. A fixed plan
+        fed column by column gives the bits of `run()` with that plan."""
+        t = self._t
+        if t is None:
+            raise RuntimeError("step() needs begin(batch) first")
+        st = self._st
+        if t >= self.T:
+            raise RuntimeError(f"step(): the rollout reached step_end={self.T}")
+        if player_action is not None:
+            if not self._players:
+                raise ValueError("step(player_action) needs a batch with player/valid")
+            st["player_action"][:, :, t].copy_(self._plan_column(player_action), non_blocking=True)
+        if self.use_graph:
+            self._graph[t % 2].replay()  # step t + 1: odd steps use graph 0
+        else:
+            self._step(st, self._static, self._navi)
+        self.graph_steps += 1
+        self._t = t + 1
+        return self._observe()
+
+    def _plan_column(self, a: Tensor) -> Tensor:
+        """[n_sc, (R,) A_caller, 2] actions -> [B, A, 2] on the device in the kept agent slots' order."""
+        st, R = self._st, self.R
+        n_sc, A = st["n_sc"], self._A_full
+        if not a.is_floating_point() or tuple(a.shape) not in ((n_sc, A, 2), (n_sc, R, A, 2)):
+            raise ValueError(f"player_action: expected float [{n_sc}, ({R},) {A}, 2], got {a.dtype} {tuple(a.shape)}")
+        if not bool(torch.isfinite(a).all()):
+            raise ValueError("player_action holds non-finite values")
+        a = a.to(self.dev, torch.float32, non_blocking=True)
+        a = a if a.dim() == 4 else a[:, None].expand(-1, R, -1, -1)
+        if self._perm is not None:
+            a = torch.gather(a, 2, self._perm[:, None, :, None].expand(-1, R, -1, 2))
+        return a.reshape(st["B"], st["A"], 2)
+
+    def _observe(self) -> Dict[str, Tensor]:
+        st = self._st
+        out = dict(valid=st["valid"].bool(), pose=st["pose"].clone(), motion=st["motion"].clone())
+        if self._perm is not None:
+            out = {k: self._caller_order(v) for k, v in out.items()}
+        out["t"] = self._t
+        return out
+
+    def _caller_order(self, t: Tensor) -> Tensor:
+        """[n_sc*R, A_kept, ...] -> [n_sc*R, A, ...] in the caller's agent order; dropped slots read as zeros."""
+        n_sc, R, A = self._st["n_sc"], self.R, self._A_full
+        sc = torch.arange(n_sc, device=self.dev)[:, None]
+        full = t.new_zeros((n_sc, R, A) + tuple(t.shape[2:]))
+        full[sc, :, self._perm] = t.view((n_sc, R, -1) + tuple(t.shape[2:])).transpose(1, 2)
+        return full.view((n_sc * R, A) + tuple(t.shape[2:]))
+
     def results(self) -> Dict[str, Tensor]:
         st, R = self._st, self.R
         n_sc, A = st["n_sc"], st["A"]
@@ -592,14 +728,7 @@ class RolloutEngine:
                    final_valid=st["valid"].bool(), final_navi_valid=~st["navi_invalid"])
         if self._perm is not None:  # back to the caller's agent order; the dropped (never valid) slots read as zeros
             A = self._A_full
-            sc = torch.arange(n_sc, device=self.dev)[:, None]
-
-            def scatter(t):
-                full = t.new_zeros((n_sc, R, A) + tuple(t.shape[2:]))
-                full[sc, :, self._perm] = t.view((n_sc, R, -1) + tuple(t.shape[2:])).transpose(1, 2)
-                return full.view((n_sc * R, A) + tuple(t.shape[2:]))
-
-            out = {k: scatter(v) for k, v in out.items()}
+            out = {k: self._caller_order(v) for k, v in out.items()}
         out["tl_state"] = tl.bool()
         out["joint_pose"] = out["pred_pose"].view(n_sc, R, A, self.T, 3)
         return out

@@ -23,7 +23,7 @@ EXPORTS = ["tb_strerror", "tb_version", "tb_knn_select", "tb_knarpe_attn", "tb_l
            "tb_traj_global", "tb_womd_post", "tb_ag_frontend", "tb_ag_frontend_blob_halves", "tb_knarpe_attn_bwd", "tb_set_fp16_flag", "tb_dyn_step_ex", "tb_tl_step_ex",
            "tb_dyn_update", "tb_chain_program_bytes", "tb_chain_encode", "tb_chain_run", "tb_layernorm_bwd", "tb_linear_wgrad", "tb_grad_mask",
            "tb_group_sum", "tb_pointnet_pool_bwd", "tb_il_loss_fwd", "tb_il_loss_bwd", "tb_tl_nll", "tb_softmax_nll", "tb_ag_featurize_ex",
-           "tb_tl_featurize_ex", "tb_colsum", "tb_ag_frontend_ex", "tb_tf32_split3"]
+           "tb_tl_featurize_ex", "tb_colsum", "tb_ag_frontend_ex", "tb_tf32_split3", "tb_dyn_step_player"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -99,6 +99,8 @@ def load() -> ctypes.CDLL:
                         I, P, P, P, P, P, P, P],
         "tb_dyn_step_ex": [P, P, P, P, F, P, P, P, P, P, P, P, P, P, P, I, I, P, P, P, P, P, P, I, I, F, F, F, P, I, I,
                            I, I, P, P, P, P, P, P, P, P, P],
+        "tb_dyn_step_player": [P, P, P, P, F, P, P, P, P, P, P, P, P, P, P, I, I, P, P, P, P, P, P, I, I, F, F, F, P, I,
+                               I, I, I, P, P, P, P, P, P, P, P, P, P, P],
         "tb_tl_step": [P, P, P, I, P, I, I, I, I, P, P, P],
         "tb_tl_step_ex": [P, P, P, I, P, I, I, I, I, P, P, P, P],
         "tb_dyn_update": [P, P, P, P, P, P, P, F, I, P, P, P, P, P, P],
