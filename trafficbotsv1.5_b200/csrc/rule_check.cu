@@ -12,8 +12,10 @@
 
 namespace {
 
+// tests/_rule_scenes.py mirrors MAX_A and QCAP: its crowd and dense-map scenes overflow both queues (more than QCAP
+// agent pairs / (polyline, vehicle) pairs), so the inline fallbacks run under test.
 constexpr int MAX_A = 256;
-constexpr int QCAP = 4096;  // (polyline, agent) candidate queue per rollout-scene
+constexpr int QCAP = 4096;  // candidate queue per rollout-scene: agent pairs, then (polyline, vehicle) pairs
 enum : unsigned { F_COL = 1, F_WOSAC = 2, F_EDGE = 4, F_RED = 8, F_LANE = 16, F_TLAHEAD = 32, F_AGAHEAD = 64 };
 
 struct Args {

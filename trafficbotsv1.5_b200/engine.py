@@ -404,7 +404,7 @@ class RolloutEngine:
                 L.ptr(tlp["tl_token_pose"]), L.ptr(st["seg"]), L.ptr(st["node_invalid"]), L.ptr(st["poly_circle"]),
                 L.ptr(st["poly_kind"]), st["n_mp"], st["n_node"], L.ptr(st["passive_counter"]),
                 *[L.ptr(st[f"vio_{k}"]) for k in VIOLATIONS], L.ptr(st["d_step"]), st["B"], st["A"], self.T, m.W,
-                st["n_tl"], self.R, self.R, 1.1, L.stream()), "tb_rule_check")
+                st["n_tl"], self.R, self.R if self.tl_per_scene else 1, 1.1, L.stream()), "tb_rule_check")  # hist_tl: Bt rows
             ops._count()
         L.check(lib.tb_step_advance(L.ptr(st["d_step"]), L.stream()), "tb_step_advance")
         L.check(lib.tb_step_advance(L.ptr(st["d_step_tl"]), L.stream()), "tb_step_advance")
