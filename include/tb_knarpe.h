@@ -447,6 +447,28 @@ int tb_rule_check(const uint8_t* pred_valid, const float* pred_pose, const float
 /* s <- s + 1 on the device (single thread); keeps the step graph replayable. */
 int tb_step_advance(int* d_step, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Batched row copy (csrc/state_copy.cu): the rollout engine's snapshot / restore / fork of its device state in one
+ * launch. Item i copies n_rows rows of row_bytes bytes from src to dst (both dense). With `src_rollout` (int32, one
+ * entry per row of the longest per-rollout item) every item with per_rollout != 0 is a row gather over the R rollouts
+ * of a scene: row b = sc * R + r of dst receives row sc * R + src_rollout[b] of src; an entry outside [0, R) copies
+ * row b itself (defined, never an out-of-range read). Other items, and all items when src_rollout is NULL, are plain
+ * copies. Accesses are 16 bytes wide where src, dst and row_bytes allow it, narrower otherwise. Items must not
+ * overlap each other. The item table travels in the kernel parameters: no allocation, no synchronisation.
+ * Errors: items / src / dst NULL -> TB_ERR_NULL; n_items outside 1..TB_COPY_ROWS_MAX, row_bytes or n_rows <= 0, a
+ * per-rollout item with R <= 0 or n_rows not a multiple of R -> TB_ERR_BAD_SHAPE; a gathered item with src == dst
+ * (rows would be overwritten before they are read) or of 2^32 access units or more -> TB_ERR_UNSUPPORTED.
+ * ------------------------------------------------------------------------------------------------- */
+#define TB_COPY_ROWS_MAX 64
+typedef struct tb_row_copy_t {
+  const void* src;
+  void* dst;
+  long long row_bytes;
+  int n_rows;
+  int per_rollout;
+} tb_row_copy_t;
+int tb_copy_rows(const tb_row_copy_t* items, int n_items, const int32_t* src_rollout, int R, void* stream);
+
 /* Gather rows: out[m, 0:C] = table[(m / rows_per_batch / div) * T + idx[m], 0:C] — navigation.py:69,
  * traffic_light.py:115. */
 int tb_gather_rows(const float* table, int ldt, int T, const int32_t* idx, int M, int rows_per_batch, int div, int C,

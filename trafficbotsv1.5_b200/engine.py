@@ -87,6 +87,17 @@ def _copy_tree(dst, src) -> None:
             x.copy_(y)
 
 
+class RolloutSnapshot:
+    """The stepped state of a rollout engine at time `t` (see `RolloutEngine.snapshot`); opaque to callers."""
+
+    def __init__(self, t: int, host_step: int, gen: int, bufs: Dict[str, Tensor]):
+        self.t, self._host_step, self._gen, self._bufs = t, host_step, gen, bufs
+
+    @property
+    def nbytes(self) -> int:
+        return sum(b.numel() * b.element_size() for b in self._bufs.values())
+
+
 class RolloutEngine:
     def __init__(self, P: Dict[str, Tensor], cfg: Optional[dict] = None, device="cuda", precision: int = 0,
                  n_rollout: int = 32, step_end: Optional[int] = None, use_graph: bool = True,
@@ -126,6 +137,7 @@ class RolloutEngine:
         self._graphs = {}
         self._players = False  # the prepared batch has player-controlled agents
         self._t = None       # current time of step-by-step stepping (begin / step); None: not begun
+        self._gen = 0        # generation of the prepared batch: a snapshot restores only into the batch it was taken of
         self._host_step = 1  # parity source for eager _step calls
         self._shape = None
         self._side = torch.cuda.Stream(device=self.dev)  # traffic-light branch runs beside the agent front-end
@@ -560,6 +572,7 @@ class RolloutEngine:
         and "tf/forcing_agent" (log replay: these agents follow their ground truth wherever it is valid)."""
         batch = self._compact(self._player_inputs(batch))
         self._players, self._t = "player/valid" in batch, None
+        self._gen += 1
         n_sc, A, n_gt = batch["sc/ag_valid"].shape
         n_tl = batch["sc/tl_valid"].shape[1]
         _, n_mp, n_node = batch["sc/mp_valid"].shape
@@ -686,6 +699,70 @@ class RolloutEngine:
         self.graph_steps += 1
         self._t = t + 1
         return self._observe()
+
+    # ---------------------------------------------------------------------------------------------- snapshot / fork
+    def _state_items(self):
+        """Everything a policy step writes that a later step reads, as (name, tensor, per_rollout). Per-rollout rows
+        (n_sc * R) follow a fork map; per-scene rows and the loop counters are copied as they are. Not included: what
+        `prepare` fixes (latent, destination, navigation / latent static features, ag_attr / ag_type, player_valid,
+        teacher-forcing tables, map) and per-step scratch (x_cat, the heads' cat buffer), written before it is read."""
+        st = self._st
+        per_rollout = ["valid", "disabled", "navi_invalid", "dest_reached", "pose", "motion", "hist_valid", "hist_pose",
+                       "hist_motion", "pred_valid", "pred_pose", "pred_motion", "knn_state", "knn_state_tl"]
+        if self._players:
+            per_rollout.append("player_action")  # step(action) writes its column
+        if self.rule_checks:
+            per_rollout += ["passive_counter"] + [f"vio_{k}" for k in VIOLATIONS]
+        if self.record_feedback:
+            per_rollout += ["fb_outside", "fb_reached"]
+        items = [(k, st[k], True) for k in per_rollout]
+        # per scene: TL ring / outputs and both buffer sets of the software-pipelined TL branch; the loop counters
+        per_scene = ["hist_tl", "tl_out"] + (["tl_nll"] if self.record_feedback else []) + ["tl_feat", "tl_logits"]
+        items += [(k, st[k], False) for k in per_scene]
+        items += [(f"kv_tl.{p}.{i}", t, False) for p, tabs in enumerate(st["kv_tl"]) for i, t in enumerate(tabs)]
+        items += [("d_step", st["d_step"], False), ("d_step_tl", st["d_step_tl"], False)]
+        return items
+
+    def snapshot(self) -> "RolloutSnapshot":
+        """Copy the rollout state at the current time of step-by-step stepping into fresh device tensors (one
+        tb_copy_rows launch, stream ordered). Several snapshots may be held at once; `restore` returns to any of them
+        while the same prepared batch is loaded."""
+        if self._t is None:
+            raise RuntimeError("snapshot() needs begin(batch) first")
+        items = self._state_items()
+        bufs = [torch.empty_like(t) for _, t, _ in items]
+        ops.copy_rows([(t, b, False) for (_, t, _), b in zip(items, bufs)])
+        return RolloutSnapshot(self._t, self._host_step, self._gen, {k: b for (k, _, _), b in zip(items, bufs)})
+
+    def restore(self, snap: "RolloutSnapshot", src: Optional[Tensor] = None) -> Dict[str, Tensor]:
+        """Write a snapshot back into the state buffers the captured step graphs read (in place, one launch, nothing is
+        re-captured) and set the time back to the snapshot's. `src` [n_sc, R] (integer): rollout r of scene sc resumes
+        from rollout src[sc, r] of the snapshot, e.g. `best[:, None].expand(-1, R)` forks the committed branch into all
+        R. Only the stepped state moves: a rollout keeps its own latent, destination and player flag. Returns the
+        observation at the snapshot's time (see `step`)."""
+        if getattr(self, "_st", None) is None:
+            raise RuntimeError("restore() needs a prepared batch")
+        if not isinstance(snap, RolloutSnapshot):
+            raise TypeError(f"restore(): expected a RolloutSnapshot, got {type(snap).__name__}")
+        if snap._gen != self._gen:
+            raise RuntimeError("restore(): the snapshot was taken of another prepared batch")
+        fork = None if src is None else self._fork_map(src)
+        items = self._state_items()
+        ops.copy_rows([(snap._bufs[k], t, pr) for k, t, pr in items], fork, self.R)
+        self._t, self._host_step = snap.t, snap._host_step
+        return self._observe()
+
+    def _fork_map(self, src: Tensor) -> Tensor:
+        """Validate a fork map on the host; returns it as int32 [n_sc * R] on the device."""
+        n_sc, R = self._st["n_sc"], self.R
+        if not isinstance(src, Tensor) or src.is_floating_point() or src.is_complex() or src.dtype == torch.bool:
+            raise ValueError(f"restore(src=...): expected an integer tensor, got {getattr(src, 'dtype', type(src))}")
+        if tuple(src.shape) != (n_sc, R):
+            raise ValueError(f"restore(src=...): expected shape [{n_sc}, {R}], got {tuple(src.shape)}")
+        h = src.detach().to("cpu", torch.int64)
+        if bool((h < 0).any()) or bool((h >= R).any()):
+            raise ValueError(f"restore(src=...): rollout indices must lie in [0, {R})")
+        return h.to(torch.int32).reshape(-1).to(self.dev)
 
     def _plan_column(self, a: Tensor) -> Tensor:
         """[n_sc, (R,) A_caller, 2] actions -> [B, A, 2] on the device in the kept agent slots' order."""

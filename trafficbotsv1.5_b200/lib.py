@@ -14,7 +14,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_PKG)
 SO_PATH = os.environ.get("TB_LIB", os.path.join(_PKG, "libtbknarpe.so"))
 _SOURCES = ["api.cu", "knn_select.cu", "knarpe_attn.cu", "knarpe_attn_mma.cu", "knarpe_attn_bwd.cu", "linear_f32.cu", "linear_tc.cu", "elementwise.cu", "post_process.cu", "ag_frontend.cu", "mlp_chain.cu",
-            "rollout_step.cu", "rule_check.cu", "train_bwd.cu", "wgrad_tc.cu"]
+            "rollout_step.cu", "rule_check.cu", "train_bwd.cu", "wgrad_tc.cu", "state_copy.cu"]
 _lib = None
 
 EXPORTS = ["tb_strerror", "tb_version", "tb_knn_select", "tb_knarpe_attn", "tb_linear", "tb_linear_ln", "tb_layernorm",
@@ -23,7 +23,7 @@ EXPORTS = ["tb_strerror", "tb_version", "tb_knn_select", "tb_knarpe_attn", "tb_l
            "tb_traj_global", "tb_womd_post", "tb_ag_frontend", "tb_ag_frontend_blob_halves", "tb_knarpe_attn_bwd", "tb_set_fp16_flag", "tb_dyn_step_ex", "tb_tl_step_ex",
            "tb_dyn_update", "tb_chain_program_bytes", "tb_chain_encode", "tb_chain_run", "tb_layernorm_bwd", "tb_linear_wgrad", "tb_grad_mask",
            "tb_group_sum", "tb_pointnet_pool_bwd", "tb_il_loss_fwd", "tb_il_loss_bwd", "tb_tl_nll", "tb_softmax_nll", "tb_ag_featurize_ex",
-           "tb_tl_featurize_ex", "tb_colsum", "tb_ag_frontend_ex", "tb_tf32_split3", "tb_dyn_step_player"]
+           "tb_tl_featurize_ex", "tb_colsum", "tb_ag_frontend_ex", "tb_tf32_split3", "tb_dyn_step_player", "tb_copy_rows"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -105,6 +105,7 @@ def load() -> ctypes.CDLL:
         "tb_tl_step_ex": [P, P, P, I, P, I, I, I, I, P, P, P, P],
         "tb_dyn_update": [P, P, P, P, P, P, P, F, I, P, P, P, P, P, P],
         "tb_step_advance": [P, P],
+        "tb_copy_rows": [P, I, P, I, P],
         "tb_chain_program_bytes": [],
         "tb_chain_encode": [P, I, I, P],
         "tb_chain_run": [P, P, P, I, I, P],
@@ -127,6 +128,12 @@ def load() -> ctypes.CDLL:
     lib.tb_version.restype = c_int
     _lib = lib
     return lib
+
+
+class RowCopy(ctypes.Structure):
+    """tb_row_copy_t: one buffer of a tb_copy_rows launch."""
+    _fields_ = [("src", c_void_p), ("dst", c_void_p), ("row_bytes", ctypes.c_longlong), ("n_rows", c_int),
+                ("per_rollout", c_int)]
 
 
 def check(code: int, what: str) -> None:

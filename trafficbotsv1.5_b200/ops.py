@@ -264,6 +264,22 @@ def gather_rows(table: Tensor, idx: Tensor, rows_per_batch: int, div: int = 1, o
     return out
 
 
+def copy_rows(items, src_rollout: Optional[Tensor] = None, R: int = 0) -> None:
+    """tb_copy_rows: one launch for all `items` = [(src, dst, per_rollout)], contiguous tensors of equal shape and
+    dtype whose rows run along dim 0. With `src_rollout` (int32 [rows], on the device) the per-rollout items gather
+    row sc * R + src_rollout[b] into row b = sc * R + r; the others, and all of them without a map, are plain copies."""
+    arr = (L.RowCopy * len(items))()
+    for i, (src, dst, per_rollout) in enumerate(items):
+        assert src.shape == dst.shape and src.dtype == dst.dtype and src.is_contiguous() and dst.is_contiguous()
+        rows = src.shape[0]
+        arr[i] = L.RowCopy(src.data_ptr(), dst.data_ptr(), src.numel() * src.element_size() // rows, rows,
+                           int(per_rollout))
+    if src_rollout is not None:
+        assert src_rollout.dtype == torch.int32 and src_rollout.is_contiguous()
+    L.check(L.load().tb_copy_rows(arr, len(items), L.ptr(src_rollout), R, L.stream()), "tb_copy_rows")
+    _count()
+
+
 def host_f3(vals):
     return (ctypes.c_float * 3)(*[float(v) for v in vals])
 
