@@ -377,10 +377,22 @@ int tb_dyn_step_player(const float* act_branch, const uint8_t* ag_type, const fl
  *   kind 0 GEMM: acc[128 x 128] = A W[n0 : n0+128, :]^T with A = the 128-column buffers a_buf[0 .. K/128) side by side
  *     (K a multiple of 64, <= 512) and W [N, K] fp16 row-major (rows past N read as zero);
  *     v = acc + bias[n0 + c]; relu; if mask_pre[row]: 0; += res[row, res_col + c]; if mask_post[row]: 0 — the epilogue of
- *     tb_linear. v goes to buffer out_buf as fp16 and/or to fp32 rows out_g[row, g_col + c] (c < n_valid) and/or fp16 rows
- *     out_h[row, h_col + c]; with ln_out, fp16(LayerNorm(v) * ln_gamma + ln_beta) (eps 1e-5) goes to ln_out[row, c].
+ *     tb_linear. v goes to buffer out_buf as fp16 (all 128 columns) and/or to fp32 rows out_g[row, g_col + c] and/or
+ *     fp16 rows out_h[row, h_col + c], both for c < n_valid only (0 = 128); with ln_out, fp16(LayerNorm(v) * ln_gamma +
+ *     ln_beta) of all 128 columns (eps 1e-5) goes to ln_out[row, c]. The residual rows are read for all 128 columns.
+ *     fp16 conversions (LOAD of fp32, out_buf, out_h, ln_out) round to nearest and saturate at +-65504; a buffer or out_h
+ *     value that reaches the bound sets the tb_set_fp16_flag word.
  * bias / ln_gamma / ln_beta / W are device pointers baked into the program (model constants; bias must hold n0 + 128
- * floats); mask_pre, mask_post, res, out_g, out_h, ln_out, src are indices into the `bindings` array passed at run time.
+ * floats, ln_gamma / ln_beta 128, W / ln_gamma / ln_beta 16-byte aligned); mask_pre, mask_post, res, out_g, out_h,
+ * ln_out, src are indices into the `bindings` array passed at run time.
+ * Aliasing within one launch:
+ *   - a LOAD source is read through the non-coherent cache (ld.global.nc): no unit of the launch may write what a LOAD
+ *     reads. tb_chain_run refuses (TB_ERR_UNSUPPORTED) a LOAD whose binding pointer is also an out_g / out_h / ln_out
+ *     binding unless both have the same row pitch and disjoint column ranges inside one row.
+ *   - residual rows are read with plain loads, by the thread that owns the row slice [32 q, 32 q + 32) of the unit, so a
+ *     residual may read what an EARLIER unit of the launch wrote through out_g at the same binding, leading dimension and
+ *     column offset (the head chain: add_latent reads add_navi's output this way). Two units that touch the same global
+ *     element must use the same binding, leading dimension and column offset; other overlaps race.
  * ------------------------------------------------------------------------------------------------- */
 #define TB_CHAIN_MAX_UNITS 32
 #define TB_CHAIN_MAX_KB 8
@@ -399,9 +411,21 @@ typedef struct tb_chain_unit {
 } tb_chain_unit;
 int tb_chain_program_bytes(void);
 /* host_blob: tb_chain_program_bytes() bytes of host memory; copy it to 128-byte aligned device memory afterwards.
- * n_buf: on-chip activation buffers (2..6; the rest of the 227 KB of shared memory is the weight ring). */
+ * n_buf: on-chip activation buffers, 2..5 (else TB_ERR_BAD_SHAPE). The rest of the 227 KB of shared memory is the weight
+ * ring: (227 KB - 1 KB - 32 KB n_buf - 704 n_units - 4928) / 16 KB stages, at most 8, i.e.
+ *   n_buf 2: 8 | 3: 7 (1-19 units), 6 (20-32) | 4: 5, 4 | 5: 3, 2 — n_stage, the 4th int of the host blob.
+ * A GEMM unit waits for the last writer of each of its (at most 4) input buffers and, from the 5th GEMM on, for the
+ * epilogue of the GEMM 4 earlier (the 4 TMEM accumulator regions are used in turn): at most 5 waits.
+ * Errors: n_units outside 1..32, n_buf outside 2..5, out_buf >= n_buf, a binding index outside -1..14, a misshapen LOAD
+ * (lds / src_col not multiples of 4 (fp32) or 8 (fp16)) or GEMM (K not a multiple of 64 or > 512, n0 >= N, n_valid
+ * > 128), reading a buffer nobody wrote -> TB_ERR_BAD_SHAPE; misaligned W / bias / ln_gamma / ln_beta, ldr / res_col
+ * not multiples of 4, ldh / h_col / ld_ln not multiples of 8, ln_out without gamma / beta -> TB_ERR_MISALIGNED; more than
+ * 24 distinct (W, K, N) weights -> TB_ERR_UNSUPPORTED. All of these are returned before any device work. */
 int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_buf, void* host_blob);
-/* bindings: HOST array of n_bind (<= 15) device pointers. Rows >= M of the last tile are neither read nor written. */
+/* bindings: HOST array of n_bind (<= 15) device pointers. Rows >= M of the last tile are neither read nor written.
+ * Before the launch every binding the program uses is checked: index >= n_bind -> TB_ERR_BAD_SHAPE, NULL -> TB_ERR_NULL,
+ * base not 16-byte aligned (LOAD sources, residual, out_h, ln_out, out_g with (ldg | g_col) % 4 == 0) or 4-byte aligned
+ * (other out_g) -> TB_ERR_MISALIGNED, a LOAD source written by the launch (see Aliasing) -> TB_ERR_UNSUPPORTED. */
 int tb_chain_run(const void* d_program, const void* host_blob, void* const* bindings, int n_bind, int M, void* stream);
 
 /* Traffic-light feedback — utils/dynamics.py:144-163 (override_tl), traffic_light.py:286 (clamp +-3).

@@ -32,6 +32,7 @@ constexpr int EPI_WARPS = 16;
 constexpr int NUM_THREADS = (EPI_WARPS + 2) * 32;
 constexpr int MAX_UNITS = TB_CHAIN_MAX_UNITS;
 constexpr int MAX_MAPS = 24;
+constexpr int MAX_BUF = 5;
 constexpr int SMEM_MAX = 227 * 1024;
 
 // Device-side unit record (192 bytes, staged in shared memory). The fields a warp needs on its critical path sit in
@@ -370,10 +371,16 @@ mlp_chain_kernel(const uint8_t* __restrict__ prog, const Bind bind, int M) {
             for (int j = 0; j < 32; ++j) v[j] = 0.f;
           }
         }
+        const int nv = hq.w - cq * 32;  // columns of this slice that exist for out_g / out_h (< 32: narrow output)
         if (flags & (F_OBUF | F_OH)) {
           uint32_t h[16], hm = 0u;
 #pragma unroll
           for (int j = 0; j < 16; ++j) { h[j] = tb_pack_h2_sat(v[2 * j], v[2 * j + 1]); tb_track_h2(hm, h[j]); }
+          if (!(flags & F_OBUF) && nv < 32) {  // only out_h's c < n_valid are stored: only they can raise the flag
+            hm = 0u;
+#pragma unroll
+            for (int j = 0; j < 16; ++j) tb_track_h2(hm, 2 * j + 1 < nv ? h[j] : 2 * j < nv ? (h[j] & 0xFFFFu) : 0u);
+          }
           if (flags & F_OBUF) {  // fp16 row slice -> the next A operand (K-major, 128-byte swizzle)
             const uint32_t kb_base = act_s + (uint32_t)hq.z + (uint32_t)kblk * KB_BYTES;
 #pragma unroll
@@ -384,16 +391,21 @@ mlp_chain_kernel(const uint8_t* __restrict__ prog, const Bind bind, int M) {
           if ((flags & F_OH) && rok) {
             __half* hp = static_cast<__half*>(bptr(lds32(ua + UOFF(out_h)))) + (size_t)grow * lds32(ua + UOFF(ldh)) +
                          lds32(ua + UOFF(h_col)) + cq * 32;
+            if (nv >= 32) {
 #pragma unroll
-            for (int c = 0; c < 4; ++c)
-              *reinterpret_cast<uint4*>(hp + 8 * c) = make_uint4(h[4 * c], h[4 * c + 1], h[4 * c + 2], h[4 * c + 3]);
+              for (int c = 0; c < 4; ++c)
+                *reinterpret_cast<uint4*>(hp + 8 * c) = make_uint4(h[4 * c], h[4 * c + 1], h[4 * c + 2], h[4 * c + 3]);
+            } else {
+#pragma unroll
+              for (int j = 0; j < 32; ++j)
+                if (j < nv) hp[j] = __ushort_as_half((unsigned short)(h[j >> 1] >> (16 * (j & 1))));
+            }
           }
           if (rok) tb_flag_if_sat(hm, static_cast<unsigned int*>(bptr(TB_CHAIN_MAX_BIND - 1)));
         }
         if ((flags & F_OG) && rok) {
           const int ldg = lds32(ua + UOFF(ldg)), gcol = lds32(ua + UOFF(g_col));
           float* gp = static_cast<float*>(bptr(lds32(ua + UOFF(out_g)))) + (size_t)grow * ldg + gcol + cq * 32;
-          const int nv = hq.w - cq * 32;  // columns of this slice that exist
           if (nv >= 32 && ((ldg | gcol) & 3) == 0) {
 #pragma unroll
             for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(gp + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
@@ -471,6 +483,54 @@ int tail_bytes(int n_units) {
 
 size_t blob_bytes() { return 64 + ((sizeof(UnitDev) * MAX_UNITS + 63) & ~(size_t)63) + (size_t)MAX_MAPS * 128; }
 
+// The bindings a program uses, checked from the host copy of the program before any launch: every index is below
+// n_bind (else TB_ERR_BAD_SHAPE), not NULL (TB_ERR_NULL) and aligned for the widest access the kernel makes through it
+// (TB_ERR_MISALIGNED): 16 bytes for LOAD sources (ldg4 / uint4), residual rows (float4), out_h and ln_out rows (uint4)
+// and out_g rows with (ldg | g_col) % 4 == 0 (float4), 4 bytes for other out_g rows. LOAD sources are read through the
+// non-coherent path (ld.global.nc), so a LOAD whose binding (same pointer) is also written by the launch through out_g /
+// out_h / ln_out is refused (TB_ERR_UNSUPPORTED) unless both rows have the same pitch in bytes and their column byte
+// ranges lie inside one row and do not overlap (the head chain reads the right half of the buffer it writes the left
+// half of).
+int check_bindings(const UnitDev* units, int n_units, void* const* bindings, int n_bind) {
+  auto need = [&](int i, uintptr_t align) {
+    if (i < 0 || i >= n_bind) return TB_ERR_BAD_SHAPE;
+    if (!bindings[i]) return TB_ERR_NULL;
+    return (reinterpret_cast<uintptr_t>(bindings[i]) & (align - 1)) ? TB_ERR_MISALIGNED : TB_OK;
+  };
+  for (int u = 0; u < n_units; ++u) {
+    const UnitDev& d = units[u];
+    int e = TB_OK;
+    if (d.flags & F_LOAD) {
+      if ((e = need(d.src, 16))) return e;
+      continue;
+    }
+    if ((d.flags & F_MPRE) && (e = need(d.mask_pre, 1))) return e;
+    if ((d.flags & F_MPOST) && (e = need(d.mask_post, 1))) return e;
+    if ((d.flags & F_RES) && (e = need(d.res, 16))) return e;
+    if ((d.flags & F_OG) && (e = need(d.out_g, ((d.ldg | d.g_col) & 3) ? 4 : 16))) return e;
+    if ((d.flags & F_OH) && (e = need(d.out_h, 16))) return e;
+    if ((d.flags & F_LN) && (e = need(d.ln_out, 16))) return e;
+  }
+  for (int u = 0; u < n_units; ++u) {
+    const UnitDev& l = units[u];
+    if (!(l.flags & F_LOAD)) continue;
+    const long es = (l.flags & F_SRC16) ? 2 : 4, pitch = l.lds * es, lo = l.src_col * es, hi = lo + 128 * es;
+    for (int v = 0; v < n_units; ++v) {
+      const UnitDev& g = units[v];
+      if (g.flags & F_LOAD) continue;
+      const struct { int flag, idx; long pitch, lo, hi; } outs[3] = {
+          {F_OG, g.out_g, g.ldg * 4L, g.g_col * 4L, (g.g_col + (long)g.n_valid) * 4L},
+          {F_OH, g.out_h, g.ldh * 2L, g.h_col * 2L, (g.h_col + (long)g.n_valid) * 2L},
+          {F_LN, g.ln_out, g.ld_ln * 2L, 0L, 256L}};
+      for (const auto& o : outs)
+        if ((g.flags & o.flag) && bindings[o.idx] == bindings[l.src] &&
+            !(o.pitch == pitch && hi <= pitch && o.hi <= pitch && (hi <= o.lo || o.hi <= lo)))
+          return TB_ERR_UNSUPPORTED;
+    }
+  }
+  return TB_OK;
+}
+
 }  // namespace
 
 extern "C" int tb_chain_program_bytes(void) { return (int)blob_bytes(); }
@@ -479,7 +539,8 @@ extern "C" int tb_chain_program_bytes(void) { return (int)blob_bytes(); }
 // device memory and passes that to tb_chain_run. Validates buffer hazards it can see statically.
 extern "C" int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_buf, void* host_blob) {
   if (!units || !host_blob) return TB_ERR_NULL;
-  if (n_units <= 0 || n_units > MAX_UNITS || n_buf < 2 || n_buf > 6) return TB_ERR_BAD_SHAPE;
+  // 6 buffers would leave (227 KB - 1 KB - 192 KB - tail) / 16 KB = 1 weight stage even for one unit: 2..5 only
+  if (n_units <= 0 || n_units > MAX_UNITS || n_buf < 2 || n_buf > MAX_BUF) return TB_ERR_BAD_SHAPE;
   EncodeTiledFn enc = get_encode();
   if (!enc) return TB_ERR_CUDA;
   uint8_t* blob = static_cast<uint8_t*>(host_blob);
@@ -494,7 +555,8 @@ extern "C" int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_bu
   hd->n_units = n_units; hd->n_buf = n_buf; hd->n_stage = n_stage > 8 ? 8 : n_stage;
   int n_maps = 0, n_gemm = 0, total_boxes = 0;
   const void* map_w[MAX_MAPS];
-  int writer[8];       // unit that last wrote every activation buffer (-1: nobody yet)
+  int map_k[MAX_MAPS], map_n[MAX_MAPS];
+  int writer[8];      // unit that last wrote every activation buffer (-1: nobody yet)
   int gemm_unit[MAX_UNITS];
   for (int b = 0; b < 8; ++b) writer[b] = -1;
   for (int u = 0; u < n_units; ++u) {
@@ -518,15 +580,18 @@ extern "C" int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_bu
     if (s.kind == 1) {  // LOAD
       if (s.src < 0 || s.out_buf < 0 || (s.src_f16 ? (s.lds | s.src_col) & 7 : (s.lds | s.src_col) & 3)) return TB_ERR_BAD_SHAPE;
     } else if (s.kind == 0) {
-      if (!s.W || s.K <= 0 || (s.K & 63) || s.K / 64 > TB_CHAIN_MAX_KB || s.N <= 0 || s.n0 < 0 || s.n0 >= s.N)
+      if (!s.W || s.K <= 0 || (s.K & 63) || s.K / 64 > TB_CHAIN_MAX_KB || s.N <= 0 || s.n0 < 0 || s.n0 >= s.N ||
+          s.n_valid > 128)
         return TB_ERR_BAD_SHAPE;
       if (!tb_aligned16(s.W) || (s.bias && !tb_aligned16(s.bias)) || (s.res >= 0 && ((s.ldr | s.res_col) & 3)) ||
-          (s.out_h >= 0 && ((s.ldh | s.h_col) & 7)) || (s.ln_out >= 0 && ((s.ld_ln & 7) || !s.ln_gamma || !s.ln_beta)))
+          (s.out_h >= 0 && ((s.ldh | s.h_col) & 7)) ||
+          (s.ln_out >= 0 && ((s.ld_ln & 7) || !s.ln_gamma || !s.ln_beta || !tb_aligned16(s.ln_gamma) ||
+                             !tb_aligned16(s.ln_beta))))
         return TB_ERR_MISALIGNED;
       d.nk = s.K / 64;
-      int m = -1;
+      int m = -1;  // one tensor map per distinct (W, K, N): the same pointer read with another shape needs its own
       for (int i = 0; i < n_maps; ++i)
-        if (map_w[i] == s.W) m = i;
+        if (map_w[i] == s.W && map_k[i] == s.K && map_n[i] == s.N) m = i;
       if (m < 0) {
         if (n_maps == MAX_MAPS) return TB_ERR_UNSUPPORTED;
         cuuint64_t gdim[2] = {(cuuint64_t)s.K, (cuuint64_t)s.N};
@@ -537,7 +602,7 @@ extern "C" int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_bu
                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
           return TB_ERR_CUDA;
-        map_w[n_maps] = s.W;
+        map_w[n_maps] = s.W; map_k[n_maps] = s.K; map_n[n_maps] = s.N;
         m = n_maps++;
       }
       d.map = m;
@@ -545,7 +610,7 @@ extern "C" int tb_chain_encode(const tb_chain_unit* units, int n_units, int n_bu
         if (unit < 0) return true;
         for (int i = 0; i < d.n_wait; ++i)
           if (d.wait[i] == unit) return true;
-        if (d.n_wait == 6) return false;
+        if (d.n_wait == 6) return false;  // defensive: 4 input buffers + the TMEM region make at most 5 waits
         d.wait[d.n_wait++] = unit;
         return true;
       };
@@ -574,6 +639,10 @@ extern "C" int tb_chain_run(const void* d_program, const void* host_blob, void* 
   if (M <= 0 || n_bind < 0 || n_bind > TB_CHAIN_MAX_BIND - 1) return TB_ERR_BAD_SHAPE;
   if (reinterpret_cast<uintptr_t>(d_program) & 127) return TB_ERR_MISALIGNED;
   const Header* hd = static_cast<const Header*>(host_blob);
+  if (hd->n_units <= 0 || hd->n_units > MAX_UNITS) return TB_ERR_BAD_SHAPE;
+  const int err = check_bindings(reinterpret_cast<const UnitDev*>(static_cast<const uint8_t*>(host_blob) + 64),
+                                 hd->n_units, bindings, n_bind);
+  if (err != TB_OK) return err;
   Bind b;
   for (int i = 0; i < TB_CHAIN_MAX_BIND; ++i) b.p[i] = i < n_bind ? bindings[i] : nullptr;
   b.p[TB_CHAIN_MAX_BIND - 1] = tb_fp16_flag_ptr;  // fp16 range guard word (common.cuh)

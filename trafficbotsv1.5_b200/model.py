@@ -302,39 +302,45 @@ class HotPathModel:
         if not hasattr(self, "_chain"):
             self._chain = {}
         if "heads" not in self._chain:
-            d = self.d
-            hw = lambda n: self._half(n, self.P[f"{n}.weight"])  # noqa: E731
-            b = lambda n: self.P[f"{n}.bias"]  # noqa: E731
-            q = ops.ChainProgram(self.dev, n_buf=4)
-            q.load(1, d, 1)                                                                        # pe -> B1
-            q.load(0, 2 * d, 0)                                                                    # x -> B0 (used by add_navi.mlp)
-            n = "navi_encoder.mlp_pe.fc_layers.0"
-            q.gemm(hw(n), [1], b(n), res=2, ldr=d, out_buf=2)                                      # nf (navigation.py:73-79)
-            for i, (src_b, dst_b) in zip((0, 3, 6), ((2, 1), (1, 2), (2, 1))):                     # add_navi.mlp_in
-                n = f"add_navi.mlp_in.fc_layers.{i}"
-                q.gemm(hw(n), [src_b], b(n), relu=True, out_buf=dst_b, mask_post=3 if i == 6 else -1)
-            n = "add_navi.mlp.fc_layers.0"
-            q.gemm(hw(n), [0, 1], b(n), relu=True, out_buf=2)                                      # cat(x, a1)
-            n = "add_navi.mlp.fc_layers.3"
-            q.gemm(hw(n), [2], b(n), relu=True, out_buf=3)
-            n = "add_navi.mlp.fc_layers.6"
-            q.gemm(hw(n), [3], b(n), relu=True, mask_pre=3, res=0, ldr=2 * d, out_buf=0, out_g=4, ldg=2 * d)  # x2
-            q.load(4, 2 * d, 1, src_col=d)                                                         # latent feature -> B1
-            n = "add_latent.mlp.fc_layers.0"
-            q.gemm(hw(n), [0, 1], b(n), relu=True, out_buf=2)
-            n = "add_latent.mlp.fc_layers.3"
-            q.gemm(hw(n), [2], b(n), relu=True, out_buf=3)
-            n = "add_latent.mlp.fc_layers.6"
-            q.gemm(hw(n), [3], b(n), relu=True, mask_pre=5, res=4, ldr=2 * d, out_buf=0)           # x3
-            w0 = self._half("action_head.w0", self.act_w0)
-            for t in range(3):                                                                     # action_head.py:78-82
-                q.gemm(w0, [0], self.act_b0, n0=t * d, relu=True, out_buf=1 + t)
-            for t in range(3):
-                n = f"action_head.mlp_mean.{t}.fc_layers.2"
-                q.gemm(hw(n), [1 + t], b(n), relu=True, out_buf=1 + t)
-            q.gemm(self._half("action_head.w4", self.act_w4), [1, 2, 3], self.act_b4, out_g=6, ldg=6, n_valid=6)
-            self._chain["heads"] = q.finish()
+            self._chain["heads"] = self._heads_chain().finish()
         return self._chain["heads"]
+
+    def _heads_chain(self, half: bool = True):
+        """The units of `_heads_program`, not encoded. half=False keeps the fp32 weights: a description only, for a
+        float64 reference of the same program (tests/_chain_ref.py)."""
+        d = self.d
+        hw = (lambda n: self._half(n, self.P[f"{n}.weight"])) if half else (lambda n: self.P[f"{n}.weight"])  # noqa: E731
+        b = lambda n: self.P[f"{n}.bias"]  # noqa: E731
+        q = ops.ChainProgram(self.dev, n_buf=4)
+        q.load(1, d, 1)                                                                        # pe -> B1
+        q.load(0, 2 * d, 0)                                                                    # x -> B0 (used by add_navi.mlp)
+        n = "navi_encoder.mlp_pe.fc_layers.0"
+        q.gemm(hw(n), [1], b(n), res=2, ldr=d, out_buf=2)                                      # nf (navigation.py:73-79)
+        for i, (src_b, dst_b) in zip((0, 3, 6), ((2, 1), (1, 2), (2, 1))):                     # add_navi.mlp_in
+            n = f"add_navi.mlp_in.fc_layers.{i}"
+            q.gemm(hw(n), [src_b], b(n), relu=True, out_buf=dst_b, mask_post=3 if i == 6 else -1)
+        n = "add_navi.mlp.fc_layers.0"
+        q.gemm(hw(n), [0, 1], b(n), relu=True, out_buf=2)                                      # cat(x, a1)
+        n = "add_navi.mlp.fc_layers.3"
+        q.gemm(hw(n), [2], b(n), relu=True, out_buf=3)
+        n = "add_navi.mlp.fc_layers.6"
+        q.gemm(hw(n), [3], b(n), relu=True, mask_pre=3, res=0, ldr=2 * d, out_buf=0, out_g=4, ldg=2 * d)  # x2
+        q.load(4, 2 * d, 1, src_col=d)                                                         # latent feature -> B1
+        n = "add_latent.mlp.fc_layers.0"
+        q.gemm(hw(n), [0, 1], b(n), relu=True, out_buf=2)
+        n = "add_latent.mlp.fc_layers.3"
+        q.gemm(hw(n), [2], b(n), relu=True, out_buf=3)
+        n = "add_latent.mlp.fc_layers.6"
+        q.gemm(hw(n), [3], b(n), relu=True, mask_pre=5, res=4, ldr=2 * d, out_buf=0)           # x3
+        w0 = self._half("action_head.w0", self.act_w0) if half else self.act_w0
+        for t in range(3):                                                                     # action_head.py:78-82
+            q.gemm(w0, [0], self.act_b0, n0=t * d, relu=True, out_buf=1 + t)
+        for t in range(3):
+            n = f"action_head.mlp_mean.{t}.fc_layers.2"
+            q.gemm(hw(n), [1 + t], b(n), relu=True, out_buf=1 + t)
+        w4 = self._half("action_head.w4", self.act_w4) if half else self.act_w4
+        q.gemm(w4, [1, 2, 3], self.act_b4, out_g=6, ldg=6, n_valid=6)
+        return q
 
     @property
     def ln_fused(self) -> bool:

@@ -379,11 +379,14 @@ class _ChainUnit(ctypes.Structure):
 class ChainProgram:
     """Builder / runner of a fused MLP chain (tb_chain_encode / tb_chain_run): `load` and `gemm` append units,
     `finish` encodes the program (TMA descriptors of the weights included) and uploads it, `run` launches it on a set of
-    binding tensors. Weights are fp16 [N, K] row-major device tensors kept alive by the program."""
+    binding tensors. Weights are fp16 [N, K] row-major device tensors kept alive by the program.
+    `spec` keeps every unit as a plain dict of the builder's arguments (weights, biases and LayerNorm parameters as the
+    tensors given), so a reference can run the same program (tests/_chain_ref.py). A program that is only described
+    (never finished) may hold weights of any float dtype on any device."""
 
     def __init__(self, device, n_buf: int = 4):
         self.dev, self.n_buf = torch.device(device), n_buf
-        self.units, self.keep = [], []
+        self.units, self.keep, self.spec = [], [], []
         self.blob = self.host = None
 
     def _unit(self, **kw) -> _ChainUnit:
@@ -399,14 +402,21 @@ class ChainProgram:
 
     def load(self, src: int, lds: int, out_buf: int, src_col: int = 0, f16: bool = False) -> None:
         self._unit(kind=1, src=src, lds=lds, src_col=src_col, src_f16=int(f16), out_buf=out_buf)
+        self.spec.append(dict(kind="load", src=src, lds=lds, out_buf=out_buf, src_col=src_col, f16=bool(f16)))
 
     def gemm(self, w: Tensor, a_bufs, bias: Optional[Tensor] = None, n0: int = 0, relu: bool = False, out_buf: int = -1,
              mask_pre: int = -1, mask_post: int = -1, res: int = -1, ldr: int = 0, res_col: int = 0, out_g: int = -1,
              ldg: int = 0, g_col: int = 0, n_valid: int = 0, out_h: int = -1, ldh: int = 0, h_col: int = 0, ln_out: int = -1,
              ld_ln: int = 0, ln_gamma: Optional[Tensor] = None, ln_beta: Optional[Tensor] = None) -> None:
-        assert w.dtype == torch.float16 and w.is_contiguous() and w.is_cuda and w.dim() == 2
+        """w [N, K]: K columns from the buffers a_bufs side by side, 128 per buffer (the last one may contribute only
+        its first 64 columns: K = 64, 192, 320, 448)."""
+        assert w.is_contiguous() and w.dim() == 2
         N, K = w.shape
-        assert K == 128 * len(a_bufs), (w.shape, a_bufs)
+        assert len(a_bufs) == (K + 127) // 128, (w.shape, a_bufs)
+        self.spec.append(dict(kind="gemm", w=w, a_bufs=list(a_bufs), bias=bias, n0=n0, relu=bool(relu), out_buf=out_buf,
+                              mask_pre=mask_pre, mask_post=mask_post, res=res, ldr=ldr, res_col=res_col, out_g=out_g,
+                              ldg=ldg, g_col=g_col, n_valid=n_valid, out_h=out_h, ldh=ldh, h_col=h_col, ln_out=ln_out,
+                              ld_ln=ld_ln, ln_gamma=ln_gamma, ln_beta=ln_beta))
         u = self._unit(kind=0, W=w.data_ptr(), K=K, N=N, n0=n0, relu=int(relu), out_buf=out_buf, mask_pre=mask_pre,
                        mask_post=mask_post, res=res, ldr=ldr, res_col=res_col, out_g=out_g, ldg=ldg, g_col=g_col,
                        n_valid=n_valid, out_h=out_h, ldh=ldh, h_col=h_col, ln_out=ln_out, ld_ln=ld_ln)
@@ -420,11 +430,14 @@ class ChainProgram:
             self.keep.append(b)
             u.bias = b.data_ptr()
         if ln_out >= 0:
-            g, be = _f32c(ln_gamma), _f32c(ln_beta)
+            g, be = (t.detach().to(self.dev, torch.float32).contiguous() for t in (ln_gamma, ln_beta))
             self.keep += [g, be]
             u.ln_gamma, u.ln_beta = g.data_ptr(), be.data_ptr()
 
     def finish(self) -> "ChainProgram":
+        for s in self.spec:
+            assert s["kind"] == "load" or (s["w"].dtype == torch.float16 and s["w"].is_cuda), \
+                "a program that runs needs fp16 device weights"
         lib = L.load()
         n = lib.tb_chain_program_bytes()
         self.host = (ctypes.c_uint8 * n)()
