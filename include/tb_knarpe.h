@@ -156,7 +156,8 @@ int tb_tf32_split3(const float* X, int ldx, int M, int K, float* out, int ldo, v
  *   the rows the next kind::f16 projection reads, so the residual stream is not re-read by a LayerNorm launch.
  *   precision 1 (fp32 X, W) or 2 (fp16 X, W). Y, res, bias, gamma, beta 16-byte aligned, ln_out 8-byte aligned,
  *   leading dims multiples of 4; anything else: TB_ERR_UNSUPPORTED / TB_ERR_MISALIGNED (call tb_linear + tb_layernorm).
- *   Variance is E[y^2] - E[y]^2 in fp32 (one pass over the accumulator registers). */
+ *   Statistics in fp32 without cancellation: per 32 columns the sum and M2 of the values shifted by the first of them,
+ *   merged over the row with Chan's formula M2 = sum M2_h + 32 sum (mean_h - mean)^2, variance M2 / 128. */
 int tb_linear_ln(const void* X, int ldx, const void* W, const float* bias, float* Y, int ldy, int M, int N, int K,
                  const uint8_t* mask_pre, const float* res, int ldr, const uint8_t* mask_post, int precision,
                  const float* ln_gamma, const float* ln_beta, void* ln_out, int ld_ln, void* stream);

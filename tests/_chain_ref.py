@@ -171,11 +171,14 @@ def interpret(spec, bind, rows, round16=True, bound=False):
             sig = (var + 1e-5).sqrt()
             z = (v - mu) / sig
             y = z * g + be
-            # input error: mean and every column move by <= e_r, the variance by <= 2 sigma e_r + e_r^2; the kernel's
-            # one-pass fp32 statistics (sum and sum of squares of 128 values) add 2^-24 * 130 of E[v^2] to the variance
+            # input error: mean and every column move by <= e_r, the variance by <= 2 sigma e_r + e_r^2. The kernel's
+            # fp32 statistics (per 32 columns: sequential sums of v - c and (v - c)^2, c the first of them, then Chan's
+            # merge; tests/_linear_ref.ln_out_bound derives the same terms for depth-8 sums): every mean off by
+            # <= e_s = 2^-24 (130 max|v| + 470 sigma), the variance by 2^-24 3400 var + 8 sigma e_s + 8 e_s^2
             e_r = ev.amax(1, keepdim=True)
-            msq = (v * v).mean(1, keepdim=True)
-            d_var = 2 * var.sqrt() * e_r + e_r ** 2 + 2.0 ** -24 * 260 * (msq + e_r * (2 * v.abs().amax(1, keepdim=True) + e_r))
+            sd = var.sqrt() + e_r
+            e_s = 2.0 ** -24 * (130 * (v.abs().amax(1, keepdim=True) + e_r) + 470 * sd)
+            d_var = 2 * var.sqrt() * e_r + e_r ** 2 + 2.0 ** -24 * 3400 * sd ** 2 + 8 * sd * e_s + 8 * e_s ** 2
             d_mu = e_r + 2.0 ** -24 * 130 * (v.abs().mean(1, keepdim=True) + e_r)
             ey = g.abs() * ((ev + d_mu) / sig + z.abs() * d_var / (var + 1e-5)) + 2.0 ** -21 * (y.abs() + (z * g).abs())
             ey = 2 * ey + ulp16(y.abs() + 2 * ey) if round16 else 2 * ey

@@ -20,6 +20,7 @@ import pytest
 import torch
 
 import _chain_ref as CR
+import _linear_ref as LR
 from oracle import tb_oracle as O
 from trafficbotsv1_5_b200 import config, params
 
@@ -303,9 +304,9 @@ def test_engine_heads_chain_vs_oracle_and_interpreter():
     print(f"\nheads vs float64 oracle: chain {errs[True]:.2e}, per layer {errs[False]:.2e} (tolerance {tol:.1e})")
 
 
-def test_engine_ffn_program_vs_interpreter():
-    """_ffn_program (LN rows -> FFN-1 + ReLU, 4 hidden slices -> FFN-2 + residual + row mask -> fp32 rows + next
-    LayerNorm) against the interpreter on its own spec; masked rows are 0 and their LayerNorm rows exactly fp16(beta)."""
+def _ffn_run(offset=0.0):
+    """_ffn_program on 1000 seeded rows; with `offset`, every residual row is shifted by +-offset. Returns
+    (program, CPU inputs, device bindings after the run, row mask, LayerNorm gamma, LayerNorm beta)."""
     m, P, cfg = _model()
     d, M = cfg["hidden_dim"], 1000
     p, nxt = "mp_encoder.tf_mp2mp.layers.0", "mp_encoder.tf_mp2mp.layers.1.norm1"
@@ -314,14 +315,46 @@ def test_engine_ffn_program_vs_interpreter():
     mask = torch.rand(M, generator=g) < 0.3
     init = [torch.randn(M, d, generator=g).half(), torch.randn(M, d, generator=g), mask.to(torch.uint8),
             torch.full((M, d), 7.0), torch.zeros(M, d, dtype=torch.float16)]
+    if offset:
+        sign = torch.where(torch.rand(M, 1, generator=torch.Generator().manual_seed(29)) < 0.5, -1.0, 1.0)
+        init[1] += offset * sign
     out = [t.to(DEV) for t in init]
     q.run(out, M)
+    return q, init, out, mask, P[f"{nxt}.weight"], P[f"{nxt}.bias"]
+
+
+def _check_ffn(q, init, out, mask, beta):
+    M, d = init[1].shape
     X, E, _ = CR.interpret(q.spec, init, torch.arange(M), bound=True)
     for i in (3, 4):
         assert bool(((out[i].cpu().double() - X[i]).abs() <= E[i]).all()), i
     assert float(out[3][mask.to(DEV)].abs().max()) == 0.0
-    beta = P[f"{nxt}.bias"].half()
-    assert torch.equal(out[4][mask.to(DEV)].cpu(), beta.expand(int(mask.sum()), d))
+    assert torch.equal(out[4][mask.to(DEV)].cpu(), beta.half().expand(int(mask.sum()), d))
+
+
+def test_engine_ffn_program_vs_interpreter():
+    """_ffn_program (LN rows -> FFN-1 + ReLU, 4 hidden slices -> FFN-2 + residual + row mask -> fp32 rows + next
+    LayerNorm) against the interpreter on its own spec; masked rows are 0 and their LayerNorm rows exactly fp16(beta)."""
+    q, init, out, mask, _, beta = _ffn_run()
+    _check_ffn(q, init, out, mask, beta)
+
+
+def test_engine_ffn_program_layernorm_far_from_zero():
+    """The FFN program with every residual row shifted by +-1000, so the LayerNorm sees rows whose mean is hundreds of
+    times their spread: the interpreter check as above, and the fp16 LayerNorm rows against float64 LayerNorm of the
+    program's own fp32 rows within tests/_linear_ref.ln_out_bound (group sums of depth 33). A one-pass
+    E[v^2] - E[v]^2 loses the variance to cancellation here and misses that bound by orders of magnitude."""
+    q, init, out, mask, gamma, beta = _ffn_run(1000.0)
+    _check_ffn(q, init, out, mask, beta)
+    y = out[3].cpu()
+    ratio = float((y.double().mean(1).abs() / y.double().std(1).clamp_min(1e-30))[~mask].min())
+    assert ratio > 100, ratio
+    ref, _, _ = LR.layernorm_ref_f64(y, gamma, beta)
+    bound = LR.ln_out_bound(y, gamma, beta, group_depth=33)
+    err = (out[4].cpu().double() - ref).abs()
+    r = float((err / bound).max())
+    print(f"\nchain LayerNorm, mean / std >= {ratio:.0f}: worst ln_out error / bound {r:.3g}")
+    assert r <= 1.0, f"{int((err > bound).sum())} ln_out values outside the bound, worst {r:.3g} x"
 
 
 # ------------------------------------------------------------------------------------------------ refusals

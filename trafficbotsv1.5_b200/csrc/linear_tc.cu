@@ -29,7 +29,7 @@ constexpr int COLS_PER_WARP = BN / (EPI_WARPS / 4);
 constexpr int NUM_THREADS = (EPI_WARPS + 2) * 32;
 constexpr int TMEM_COLS = 2 * BN;
 constexpr int EPI_BYTES = EPI_WARPS * 32 * 32 * 4;  // one 32x32 fp32 staging block per epilogue warp
-constexpr int LN_BYTES = 2 * 4 * 4 * 32 * 8;          // fused LayerNorm: (sum, sum of squares) partials [parity][quarter][col block][row]
+constexpr int LN_BYTES = 2 * 4 * 4 * 32 * 8;          // fused LayerNorm: (sum, M2) partials [parity][quarter][col block][row]
 constexpr size_t SMEM_BYTES = 1024 /*align slack*/ + (size_t)STAGES * (A_BYTES + B_BYTES) + EPI_BYTES + LN_BYTES + 256;
 
 struct Epi {
@@ -126,6 +126,17 @@ __device__ __forceinline__ void prefetch_rows(Prefetch& pf, int rsub, int rbase,
     if (rp) rp += rstep;
   }
 }
+// Store-phase row sums: q[i] is this lane's partial of row 4 i + rsub; a butterfly over the 8 lanes of the row group
+// (7 shuffles) leaves lane (rsub, cc) with the full 32-column sum of row 4 cc + rsub.
+__device__ __forceinline__ float rowgroup_sum(const float (&q)[8], int cc) {
+  const bool b2 = cc & 4, b1 = cc & 2, b0 = cc & 1;
+  float t[4], u[2];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) t[j] = (b2 ? q[j + 4] : q[j]) + __shfl_xor_sync(TB_FULL_MASK, b2 ? q[j] : q[j + 4], 4);
+#pragma unroll
+  for (int j = 0; j < 2; ++j) u[j] = (b1 ? t[j + 2] : t[j]) + __shfl_xor_sync(TB_FULL_MASK, b1 ? t[j] : t[j + 2], 2);
+  return (b0 ? u[1] : u[0]) + __shfl_xor_sync(TB_FULL_MASK, b0 ? u[0] : u[1], 1);
+}
 template <bool RELU, bool TO_H, bool EXTRA, bool ALL, bool LN = false>
 __device__ __forceinline__ void store_block(uint32_t st_s, int rsub, int cc, int rbase, int col, int M, float4 bv,
                                             float* __restrict__ Y, int ldy, const Epi& ep, const Prefetch& pf,
@@ -171,42 +182,41 @@ __device__ __forceinline__ void store_block(uint32_t st_s, int rsub, int cc, int
   if (TO_H) tb_flag_if_sat(hmax, ep.sat_flag);
   if (LN) {
     // ---- LayerNorm of the finished rows (transformer_rpe.py:156-171, eps 1e-5): a row's 128 columns sit in the four
-    // warps of this TMEM lane quarter. Per-row (sum, sum of squares) of this warp's 32 columns by a butterfly over the
-    // 8 lanes of a row group (7 shuffles per quantity; lane (rsub, cc) ends up owning row 4 cc + rsub), partials of the
-    // four warps through shared memory + a 128-thread named barrier, statistics back to the lanes through the warp's
-    // staging block.
-    const bool b2 = cc & 4, b1 = cc & 2, b0 = cc & 1;
-    float q1[8], q2[8];
+    // warps of this TMEM lane quarter. Each warp sums its 32 columns of a row shifted by c, the row's value in the
+    // warp's first column (one broadcast from lane (rsub, 0)), and the squares of the shifted values, by a butterfly
+    // over the 8 lanes of a row group (lane (rsub, cc) ends up owning row 4 cc + rsub). c is one of the 32 values, so
+    // (mean_h - c)^2 <= M2_h and M2_h = sum (y - c)^2 - (sum (y - c))^2 / 32 loses at most a factor 33 to cancellation,
+    // whatever the row's offset. The four warps' (sum, M2) partials go through shared memory + a 128-thread named
+    // barrier and merge with Chan's formula M2 = sum M2_h + 32 sum (mean_h - mean)^2. Statistics back to the lanes
+    // through the warp's staging block.
+    float c[8], q1[8], q2[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      q1[i] = (vv[i].x + vv[i].y) + (vv[i].z + vv[i].w);
-      q2[i] = fmaf(vv[i].x, vv[i].x, fmaf(vv[i].y, vv[i].y, fmaf(vv[i].z, vv[i].z, vv[i].w * vv[i].w)));
+      c[i] = __shfl_sync(TB_FULL_MASK, vv[i].x, rsub << 3);
+      const float dx = vv[i].x - c[i], dy = vv[i].y - c[i], dz = vv[i].z - c[i], dw = vv[i].w - c[i];
+      q1[i] = (dx + dy) + (dz + dw);
+      q2[i] = fmaf(dx, dx, fmaf(dy, dy, fmaf(dz, dz, dw * dw)));
     }
-    float t1[4], t2[4], u1[2], u2[2];
+    const float w1 = rowgroup_sum(q1, cc), w2 = rowgroup_sum(q2, cc);
+    float c_own = c[0];  // the shift of the row this lane owns (row 4 cc + rsub: i = cc)
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      t1[j] = (b2 ? q1[j + 4] : q1[j]) + __shfl_xor_sync(TB_FULL_MASK, b2 ? q1[j] : q1[j + 4], 4);
-      t2[j] = (b2 ? q2[j + 4] : q2[j]) + __shfl_xor_sync(TB_FULL_MASK, b2 ? q2[j] : q2[j + 4], 4);
-    }
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      u1[j] = (b1 ? t1[j + 2] : t1[j]) + __shfl_xor_sync(TB_FULL_MASK, b1 ? t1[j] : t1[j + 2], 2);
-      u2[j] = (b1 ? t2[j + 2] : t2[j]) + __shfl_xor_sync(TB_FULL_MASK, b1 ? t2[j] : t2[j + 2], 2);
-    }
-    const float w1 = (b0 ? u1[1] : u1[0]) + __shfl_xor_sync(TB_FULL_MASK, b0 ? u1[0] : u1[1], 1);
-    const float w2 = (b0 ? u2[1] : u2[0]) + __shfl_xor_sync(TB_FULL_MASK, b0 ? u2[0] : u2[1], 1);
-    const int own = 4 * cc + rsub;  // the block row this lane now holds the 32-column sums of
+    for (int i = 1; i < 8; ++i) c_own = cc == i ? c[i] : c_own;
+    const int own = 4 * cc + rsub;  // the block row this lane now holds the 32-column (sum, M2) of
     float2* part = ln->part + (ln->parity * 4 + ln->quarter) * 4 * 32;
-    part[ln->half * 32 + own] = make_float2(w1, w2);
+    part[ln->half * 32 + own] = make_float2(fmaf(32.f, c_own, w1), fmaf(-w1, w1 * (1.f / 32.f), w2));
     asm volatile("bar.sync %0, 128;" ::"r"(1 + ln->quarter) : "memory");
-    float S1 = 0.f, S2 = 0.f;
+    float S1 = 0.f;
+#pragma unroll
+    for (int h = 0; h < 4; ++h) S1 += part[h * 32 + own].x;
+    const float mean = S1 * (1.f / BN);
+    float M2 = 0.f;
 #pragma unroll
     for (int h = 0; h < 4; ++h) {
       const float2 pp = part[h * 32 + own];
-      S1 += pp.x; S2 += pp.y;
+      const float d = fmaf(pp.x, 1.f / 32.f, -mean);
+      M2 = fmaf(32.f * d, d, M2 + pp.y);
     }
-    const float mean = S1 * (1.f / BN);
-    const float rstd = 1.f / sqrtf(fmaxf(S2 * (1.f / BN) - mean * mean, 0.f) + 1e-5f);
+    const float rstd = 1.f / sqrtf(M2 * (1.f / BN) + 1e-5f);
     __syncwarp();  // every lane has read its rows from the staging block
     asm volatile("st.shared.v2.f32 [%0], {%1,%2};" ::"r"(st_s + (uint32_t)own * 8u), "f"(mean), "f"(rstd) : "memory");
     __syncwarp();

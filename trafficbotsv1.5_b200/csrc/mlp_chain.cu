@@ -417,18 +417,28 @@ mlp_chain_kernel(const uint8_t* __restrict__ prog, const Bind bind, int M) {
         }
         if (flags & F_LN) {
           // LayerNorm of the 128-wide output row (transformer_rpe.py:156-171, eps 1e-5): this thread holds 32 of its
-          // columns, the other three warps of the lane quarter the rest -> exchange (sum, sum of squares) through smem
-          float s1 = 0.f, s2 = 0.f;
+          // columns, the other three warps of the lane quarter the rest -> exchange (sum, M2) of the 32 columns through smem
+          // and merge them with Chan's formula M2 = sum M2_q + 32 sum (mean_q - mean)^2. The 32 columns are summed
+          // shifted by their first value c: (mean_q - c)^2 <= M2_q, so sum (v - c)^2 - (sum (v - c))^2 / 32 loses at
+          // most a factor 33 to cancellation, whatever the row's offset (no E[v^2] - E[v]^2)
+          const float c = v[0];
+          float s1 = 0.f, m2 = 0.f;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) { s1 += v[j]; s2 = fmaf(v[j], v[j], s2); }
-          sLN[cq * TM + row] = make_float2(s1, s2);
+          for (int j = 0; j < 32; ++j) { const float d = v[j] - c; s1 += d; m2 = fmaf(d, d, m2); }
+          m2 = fmaf(-s1, s1 * (1.f / 32.f), m2);
+          s1 = fmaf(32.f, c, s1);
+          sLN[cq * TM + row] = make_float2(s1, m2);
           asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");
-          s1 = 0.f; s2 = 0.f;
+          float2 o[4];
+          s1 = 0.f;
 #pragma unroll
-          for (int q = 0; q < 4; ++q) { const float2 o = sLN[q * TM + row]; s1 += o.x; s2 += o.y; }
+          for (int q = 0; q < 4; ++q) { o[q] = sLN[q * TM + row]; s1 += o[q].x; }
           asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");  // partials consumed: the slots may be rewritten
           const float mean = s1 * (1.f / 128.f);
-          const float rstd = 1.f / sqrtf(fmaxf(s2 * (1.f / 128.f) - mean * mean, 0.f) + 1e-5f);
+          m2 = 0.f;
+#pragma unroll
+          for (int q = 0; q < 4; ++q) { const float d = fmaf(o[q].x, 1.f / 32.f, -mean); m2 = fmaf(32.f * d, d, m2 + o[q].y); }
+          const float rstd = 1.f / sqrtf(m2 * (1.f / 128.f) + 1e-5f);
           if (rok) {
             const float* ln_g = reinterpret_cast<const float*>(lds64(ua + UOFF(ln_g)));
             const float* ln_b = reinterpret_cast<const float*>(lds64(ua + UOFF(ln_b)));
