@@ -57,17 +57,23 @@ int tb_set_fp16_flag(unsigned int* d_flag);
  * Optional (all may be NULL / 0) — repeated selections against STATIC targets (agent -> map, every rollout step):
  *   tgt_index_map [B/div,T] int32: the targets are passed in a caller-chosen order and out_idx reports
  *     tgt_index_map[position] (ties and output order then follow the passed order);
- *   sorted_by_x != 0: the caller promises tgt_pose[..,0] ascending within each target batch;
+ *   flags & TB_KNN_SORTED_BY_X: the caller promises tgt_pose[..,0] ascending within each target batch;
  *   row_state [B,S,3] f32 (in/out): (x, y, K-th smallest squared distance) of the previous call for the same row,
  *     K-th = +inf to start. With sorted targets only the slab |x_t - x_s| <= sqrt(K-th) + |displacement| is scanned
  *     (the K nearest of the previous call still lie within that radius: same result as a full scan). Without
  *     sorted targets the state still brackets the bisection for the K-th distance. A row state REQUIRES static targets.
+ * `flags` (the former sorted_by_x argument; 1 keeps its meaning):
+ *   TB_KNN_SORTED_BY_X  the caller promises tgt_pose[..,0] ascending within each target batch (above);
+ *   TB_KNN_REFERENCE    run the previous kernels (full-length bisections, one kernel for every path) instead of the
+ *                       current ones. Both emit the same lists and row states bit for bit; kept for A/B and tests.
  * Limits: 0 < K < T <= 2048.
  * ------------------------------------------------------------------------------------------------- */
+#define TB_KNN_SORTED_BY_X 1
+#define TB_KNN_REFERENCE 2
 int tb_knn_select(const float* src_pose, const uint8_t* src_invalid, const float* tgt_pose,
                   const uint8_t* tgt_invalid, int B, int S, int T, int tgt_batch_div, int K, float dist_limit,
                   int32_t* out_idx, uint8_t* out_invalid, float* out_rel, int out_ldk, int out_koff,
-                  const int32_t* tgt_index_map, float* row_state, int sorted_by_x, void* stream);
+                  const int32_t* tgt_index_map, float* row_state, int flags, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * KNARPE attention core (gather + relative-pose bias + masked softmax + weighted sum).

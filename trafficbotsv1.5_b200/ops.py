@@ -56,9 +56,10 @@ def pe_freq_xy(pe_dim: int, theta: float = 1e3, device="cuda") -> Tensor:
 def knn_select(src_pose: Tensor, src_invalid: Tensor, tgt_pose: Tensor, tgt_invalid: Tensor, k: int,
                dist_limit: float, tgt_div: int = 1, out: Optional[Tuple[Tensor, Tensor, Tensor]] = None,
                koff: int = 0, index_map: Optional[Tensor] = None, row_state: Optional[Tensor] = None,
-               sorted_by_x: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
+               sorted_by_x: bool = False, reference: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
     """Fused get_rel_pose + get_tgt_knn_idx (utils/rpe.py:9-90). Returns idx int32 [B,S,K], invalid bool [B,S,K],
-    rel [B,S,K,3]; with `out`/`koff` writes into columns koff..koff+K of preallocated [B,S,ldk(,3)] buffers."""
+    rel [B,S,K,3]; with `out`/`koff` writes into columns koff..koff+K of preallocated [B,S,ldk(,3)] buffers.
+    reference=True runs the previous select kernels (TB_KNN_REFERENCE): the same lists and row states, bit for bit."""
     B, S, _ = src_pose.shape
     T = tgt_pose.shape[1]
     assert tgt_pose.shape[0] * tgt_div == B, (tgt_pose.shape, tgt_div, B)
@@ -77,7 +78,7 @@ def knn_select(src_pose: Tensor, src_invalid: Tensor, tgt_pose: Tensor, tgt_inva
         assert row_state.dtype == torch.float32 and row_state.is_contiguous() and row_state.shape == (B, S, 3)
     L.check(L.load().tb_knn_select(L.ptr(src_pose), L.ptr(si), L.ptr(tgt_pose), L.ptr(ti), B, S, T, tgt_div, k,
                                    float(dist_limit), L.ptr(idx), L.ptr(_u8(inv)), L.ptr(rel), ldk, koff,
-                                   L.ptr(index_map), L.ptr(row_state), int(sorted_by_x), L.stream()),
+                                   L.ptr(index_map), L.ptr(row_state), int(sorted_by_x) | (2 if reference else 0), L.stream()),
             "tb_knn_select")
     _count()
     return idx, inv, rel
